@@ -8,7 +8,10 @@ Jacobian, BASELINE.json's metric "ApplyInverse/s + HBM GB/s; GMRES solve time".
 
 A "step" is one Preconditioner::ApplyInverse on one right-hand side.  `value` is ApplyInverse/s with the vectors
 resident in HBM; `e2e` is the same call through the C ABI with pinned HOST buffers (H2D of b and D2H of x inside the
-timed region).  One JSON line is printed by rank 0.
+timed region).  One JSON line is printed by rank 0.  With --dump-outputs DIR, rank 0 also writes the vector the last
+timed ApplyInverse returned and the GMRES solution as DIR/apply_inverse_x.npy and DIR/gmres_x.npy (float64; a fixed
+sample of rows, listed in DIR/rows.npy, when they would exceed 64 MB).  The inputs depend only on the arguments, so two
+builds, or the two arms, can be compared file by file.
 
 Multi-GPU (torchrun, one rank per GPU): ONE problem ("scaling": "strong"), its subdomains distributed over the ranks
 by the reference's subdomain -> rank map (CreatePIDMap); vectors are distributed by row owner; only separator values
@@ -56,7 +59,31 @@ def parse():
                     help="grid of the cpu_baseline leg of the GPU arm (64^3: 1296 of the 9248 subdomains, ~15 s of CPU "
                          "work; its factors no longer fit the caches, like the full size)")
     ap.add_argument("--cpu-threads", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the ApplyInverse result of the last timed step (and the GMRES "
+                         "solution) as DIR/<name>.npy in float64, for comparing two builds on the same inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes each vector of `arrays` (name -> 1-D array, all of one length) as out_dir/<name>.npy in float64.  When
+    they would exceed `limit` bytes in all, every file holds the same rows: a fixed sample (numpy seed 0, ascending),
+    whose indices go to out_dir/rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    rows = None
+    if 8 * n * len(arrays) > limit - 4096:                  # (4096: room for the .npy headers)
+        k = (limit - 4096) // (8 * (len(arrays) + 1))
+        rows = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+        arrays = dict(rows=rows, **{name: np.asarray(v)[rows] for name, v in arrays.items()})
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 PARTITIONER = "Skew Cartesian"
@@ -180,7 +207,8 @@ def mem_available_gb():
 def cpu_oracle_run(nx, sx, levels, cx, steps, warmup, threads, solve):
     """The reference's CPU path restated in C++/OpenMP (oracle/cpp/hymls_oracle.cpp) on the grid `nx`: Compute,
     `steps` ApplyInverse calls, optionally the GMRES solve.  The index maps come from the library's HOST
-    partitioner (no GPU; bit-exact with oracle/partitioner.py, tests/test_host_maps.py)."""
+    partitioner (no GPU; bit-exact with oracle/partitioner.py, tests/test_host_maps.py).  Besides the figures, the
+    result holds the vectors computed: "x" (last ApplyInverse) and "gmres_x" (GMRES solution, if solved)."""
     import hymls_b200 as hb
     from oracle import cpp_oracle as oc
     from oracle.params import ParameterList
@@ -213,7 +241,7 @@ def cpu_oracle_run(nx, sx, levels, cx, steps, warmup, threads, solve):
     st = O.stats()
     out = {"nx": nx, "n": int(A.shape[0]), "subdomains": num_subdomains(nx, sx), "threads": st["threads"],
            "setup_s": t_setup, "compute_s": t_compute, "factor_a11_s": st["factor_a11_s"], "schur_s": st["schur_s"],
-           "apply_s": t_apply, "nnz_factors": st["nnz_factors"], "apply_checksum": float(np.linalg.norm(x))}
+           "apply_s": t_apply, "nnz_factors": st["nnz_factors"], "apply_checksum": float(np.linalg.norm(x)), "x": x}
     if solve:
         it = p["Solver"]["Iterative Solver"]
         xs, its, conv, hist, sec = O.solve(b, x0=x0, method="GMRES", tol=it["Convergence Tolerance"],
@@ -223,6 +251,7 @@ def cpu_oracle_run(nx, sx, levels, cx, steps, warmup, threads, solve):
                         "explicit_rel_residual": float(np.linalg.norm(A @ xs - b) / np.linalg.norm(b)),
                         "rel_error": float(np.linalg.norm(xs - xex) / np.linalg.norm(b)),
                         "history_first15": [float(v) for v in hist[:15]], "tol": it["Convergence Tolerance"]}
+        out["gmres_x"] = xs
     return out
 
 
@@ -257,6 +286,9 @@ def reference_arm(args, workload):
                             "nnz_subdomain_factors": r["nnz_factors"], "gmres": r.get("gmres")},
            "e2e": {"value": v, "unit": "1/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
            "gmres": r.get("gmres")}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v for k, v in (("apply_inverse_x", r["x"]), ("gmres_x", r.get("gmres_x")))
+                                         if v is not None})
     print(json.dumps(out))
 
 
@@ -418,6 +450,15 @@ def main():
     ms, e2e_ms, ms_a11, t_compute, solve_s = [float(v) for v in tm.cpu()]
     if gm:
         gm["solve_s"] = solve_s
+    if args.dump_outputs:
+        # the result of the last timed step, assembled from the rows each rank owns
+        x_full = torch.zeros(n, dtype=torch.float64, device="cuda")
+        x_full[torch.from_numpy(rows).cuda()] = x_own
+        if dist is not None:
+            dist.all_reduce(x_full)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"apply_inverse_x": x_full.cpu().numpy(),
+                                             **({"gmres_x": xs.cpu().numpy()} if gm else {})})
     if rank != 0:
         if dist is not None:
             dist.destroy_process_group()

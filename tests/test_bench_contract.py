@@ -1,11 +1,16 @@
 """The driver-facing contract of `bench.py --impl reference` (the CPU arm), checked without a GPU on a small grid:
 one JSON line with the metric / unit / config of the GPU arm, `impl`, `cpu_baseline` {value, unit, cores, kind, sample}
-and `e2e` {value, unit, h2d_bytes_per_step, d2h_bytes_per_step}; under torchrun only rank 0 works."""
+and `e2e` {value, unit, h2d_bytes_per_step, d2h_bytes_per_step}; under torchrun only rank 0 works.  --dump-outputs
+writes the vectors the timed path computed, in both arms (the GPU arm against the reference arm on a GPU)."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
+import bench
 from tests.conftest import ROOT
 
 
@@ -40,3 +45,58 @@ def test_reference_arm_prints_the_contract_line():
 def test_reference_arm_other_ranks_exit_without_work():
     r = _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}, "--gpus", "2", "--no-solve")
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_steps_below_one_are_rejected():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=60)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+def test_reference_arm_dumps_its_outputs(tmp_path):
+    r = _run(None, "--dump-outputs", str(tmp_path))
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert sorted(os.listdir(tmp_path)) == ["apply_inverse_x.npy", "gmres_x.npy"]
+    A, _, _, b, _ = bench.problem(32)
+    x, xs = np.load(tmp_path / "apply_inverse_x.npy"), np.load(tmp_path / "gmres_x.npy")
+    assert x.dtype == xs.dtype == np.float64 and x.shape == xs.shape == (A.shape[0],)
+    assert np.all(np.isfinite(x)) and np.linalg.norm(x) > 0
+    assert np.linalg.norm(A @ xs - b) <= 1e-7 * np.linalg.norm(b)
+
+
+def test_dump_outputs_samples_the_same_rows_of_every_vector(tmp_path):
+    n = 10000
+    v = {"a": np.arange(n, dtype=np.float64), "b": 2 * np.arange(n, dtype=np.float32)}
+    bench.dump_outputs(str(tmp_path / "full"), v)
+    assert sorted(os.listdir(tmp_path / "full")) == ["a.npy", "b.npy"]
+    assert np.array_equal(np.load(tmp_path / "full" / "a.npy"), v["a"])
+    assert np.load(tmp_path / "full" / "b.npy").dtype == np.float64
+    limit = 4096 + 3 * 8 * 1000        # room for 1000 rows of a, b and the row indices
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), v, limit=limit)
+    s1, s2 = tmp_path / "s1", tmp_path / "s2"
+    assert sum(f.stat().st_size for f in s1.iterdir()) <= limit
+    rows = np.load(s1 / "rows.npy")
+    assert len(rows) == 1000 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(s1 / "a.npy"), rows) and np.array_equal(np.load(s1 / "b.npy"), 2 * rows)
+    for name in ("rows.npy", "a.npy", "b.npy"):
+        assert np.array_equal(np.load(s1 / name), np.load(s2 / name))
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_apply_inverse_the_reference_arm_computes(tmp_path):
+    """Both arms on the same small workload: the dumped vectors are the ApplyInverse and the GMRES solution of the
+    same right-hand side.  (The bound leaves room for the rounding error of the FP64 sparse-LU reference arm; a wrong
+    or stale vector is O(1) away.)"""
+    args = ["--nx", "32", "--sx", "8", "--cx", "2", "--steps", "3", "--warmup", "1"]
+    g = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args, "--dump-outputs", str(tmp_path / "gpu")],
+                       capture_output=True, text=True, timeout=900)
+    assert g.returncode == 0, g.stderr[-2000:]
+    d = json.loads([ln for ln in g.stdout.splitlines() if ln.startswith("{")][0])
+    assert d["steps"] == 3
+    r = _run(None, "--sx", "8", "--cx", "2", "--steps", "1", "--dump-outputs", str(tmp_path / "ref"))
+    assert r.returncode == 0, r.stderr[-2000:]
+    A, _, _, b, _ = bench.problem(32)
+    xg, xr = np.load(tmp_path / "gpu" / "apply_inverse_x.npy"), np.load(tmp_path / "ref" / "apply_inverse_x.npy")
+    assert xg.shape == (A.shape[0],) and np.linalg.norm(xg - xr) <= 1e-9 * np.linalg.norm(xr)
+    assert np.linalg.norm(A @ np.load(tmp_path / "gpu" / "gmres_x.npy") - b) <= 1e-7 * np.linalg.norm(b)
