@@ -19,8 +19,6 @@
 // single-GPU path stays valid; kernels get row / group lists.
 #include <algorithm>
 #include <chrono>
-#include <cmath>
-#include <random>
 
 #include "engine.hpp"
 #include "hostpar.hpp"
@@ -344,297 +342,6 @@ int64_t Engine::ownedRows(int64_t* rows, int64_t cap) {
   if (rows && cap >= D.nOwn)
     for (int64_t i = 0; i < D.nOwn; ++i) rows[i] = D.hOwnRows[i];
   return D.nOwn;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Krylov driver on row-owner-distributed vectors (same algorithm and parameters as Engine::solve)
-// ---------------------------------------------------------------------------------------------
-void Engine::solveDist(const double* b, double* x, int where, uint64_t seed, hymls_b200_solve_info* info, double* hist,
-                       int histCap) {
-  ParameterList& sol = params_.sublist("Solver");
-  ParameterList& it = sol.sublist("Iterative Solver");
-  const std::string method = sol.get("Krylov Method", "GMRES");
-  const std::string side = sol.get("Left or Right Preconditioning", "Right");
-  const std::string startVec = sol.get("Initial Vector", "Random");
-  const int maxIters = it.get("Maximum Iterations", 1000);
-  const double tol = it.get("Convergence Tolerance", 1e-8);
-  int numBlocks = it.get("Num Blocks", 300);
-  const int maxRestarts = it.get("Maximum Restarts", 20);
-  const bool explicitTest = it.get("Explicit Residual Test", false);
-  const std::string impScaling = it.get("Implicit Residual Scaling", "Norm of Preconditioned Initial Residual");
-  const std::string expScaling = it.get("Explicit Residual Scaling", "Norm of Initial Residual");
-  Level& L0 = *levels_[0];
-  DistPlan& D = L0.dist;
-  buildMatrixHalo();
-  cudaStream_t s = stream_;
-  const int64_t n = n_, nOwn = D.nOwn, ld = (D.maxOwn + 7) & ~(int64_t)7;
-  numBlocks = std::max(1, std::min(numBlocks, maxIters));
-  const int m = numBlocks;
-  // global-length staging vectors (owned + halo entries in use) and compact vectors
-  kX_.alloc(n);   // global: argument / result of the preconditioner and the operator
-  kB_.alloc(n);   // global: second staging vector
-  kR_.alloc(ld);  // compact r
-  kW_.alloc(ld);  // compact scratch
-  kZ_.alloc(ld);  // compact scratch
-  DevBuf<double> xc, bc;  // compact solution and right-hand side
-  xc.alloc(ld);
-  bc.alloc(ld);
-  kH_.alloc(2 * m + 8);
-  kPartial_.alloc((size_t)(m + 2) * multiDotBlocks());
-  const auto kind = where == HYMLS_B200_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-  HY_CUDA(cudaMemcpyAsync(kX_.p, b, n * sizeof(double), kind, s));
-  packIdx(kX_.p, D.ownRows.p, bc.p, nOwn, s, &launches_);
-  if (startVec == "Random") {
-    std::vector<double> h(n), hc(nOwn);
-    std::mt19937_64 rng(seed);
-    for (auto& v : h) v = (double)(rng() >> 11) * (1.0 / 9007199254740992.0) * 2.0 - 1.0;
-    for (int64_t i = 0; i < nOwn; ++i) hc[i] = h[D.hOwnRows[i]];
-    HY_CUDA(cudaMemcpyAsync(xc.p, hc.data(), nOwn * sizeof(double), cudaMemcpyHostToDevice, s));
-    HY_CUDA(cudaStreamSynchronize(s));
-  } else if (startVec == "Zero") {
-    HY_CUDA(cudaMemsetAsync(xc.p, 0, ld * sizeof(double), s));
-  } else {
-    HY_CUDA(cudaMemcpyAsync(kX_.p, x, n * sizeof(double), kind, s));
-    packIdx(kX_.p, D.ownRows.p, xc.p, nOwn, s, &launches_);
-  }
-  // the ranks start the timed region together (a late rank would otherwise bill its delay to the others' first
-  // collective)
-  if (method == "GMRES") kV_.alloc((size_t)(m + 1) * ld);  // workspace (grow-only): allocated outside the timed region
-  comm_.allReduceSum(kH_.p, 1, s);
-  HY_CUDA(cudaStreamSynchronize(s));
-  HY_CUDA(cudaEventRecord(ev0_, s));
-  // operators: "global" vectors have length n with the owned entries valid
-  auto Aglobal = [&](double* full, double* outC) {  // halo of `full` is filled in place
-    haloExchange(D.mat, full, full, true);
-    spmvRows(L0.rowptr.p, L0.colidx.p, L0.val.p, full, outC, D.ownRows.p, nOwn, 0.0, nullptr, nullptr, 1.0, 1, s,
-             &launches_);
-  };
-  auto toGlobal = [&](const double* c, double* full) { scatterVec(c, D.ownRows.p, full, nOwn, s, &launches_); };
-  auto A = [&](const double* inC, double* outC) {
-    toGlobal(inC, kB_.p);
-    Aglobal(kB_.p, outC);
-  };
-  auto Mglobal = [&](const double* inC, double* outFull) {
-    toGlobal(inC, kB_.p);
-    applyLevel0Dist(kB_.p, outFull);
-    stats_.num_apply_inverse++;
-  };
-  auto M = [&](const double* inC, double* outC) {
-    Mglobal(inC, kX_.p);
-    packIdx(kX_.p, D.ownRows.p, outC, nOwn, s, &launches_);
-  };
-  auto dot = [&](const double* u, const double* v) {
-    double* d = kH_.p + 2 * m + 4;
-    multiDot(u, ld, 1, v, nOwn, kPartial_.p, d, 0, s, &launches_);
-    comm_.allReduceSum(d, 1, s);
-    double h;
-    HY_CUDA(cudaMemcpyAsync(&h, d, sizeof(double), cudaMemcpyDeviceToHost, s));
-    HY_CUDA(cudaStreamSynchronize(s));
-    return h;
-  };
-  std::vector<double> history;
-  int iters = 0;
-  bool converged = false;
-  double lastRel = 0;
-  const bool left = side == "Left", right = side == "Right";
-  const double bnorm = std::sqrt(dot(bc.p, bc.p));
-
-  if (method == "CG") {
-    DevBuf<double> P, Ap;
-    P.alloc(ld);
-    Ap.alloc(ld);
-    A(xc.p, kR_.p);
-    axpby(1.0, bc.p, -1.0, kR_.p, nOwn, s, &launches_);
-    const double r0 = std::sqrt(dot(kR_.p, kR_.p));
-    history.push_back(1.0);
-    if (r0 == 0) {
-      converged = true;
-    } else {
-      M(kR_.p, kZ_.p);
-      axpby(1.0, kZ_.p, 0.0, P.p, nOwn, s, &launches_);
-      double rz = dot(kR_.p, kZ_.p);
-      while (iters < maxIters) {
-        A(P.p, Ap.p);
-        const double alpha = rz / dot(P.p, Ap.p);
-        axpby(alpha, P.p, 1.0, xc.p, nOwn, s, &launches_);
-        axpby(-alpha, Ap.p, 1.0, kR_.p, nOwn, s, &launches_);
-        ++iters;
-        lastRel = std::sqrt(dot(kR_.p, kR_.p)) / r0;
-        history.push_back(lastRel);
-        if (lastRel <= tol) {
-          converged = true;
-          break;
-        }
-        M(kR_.p, kZ_.p);
-        const double rzNew = dot(kR_.p, kZ_.p);
-        axpby(1.0, kZ_.p, rzNew / rz, P.p, nOwn, s, &launches_);
-        rz = rzNew;
-      }
-    }
-  } else if (method == "GMRES") {
-    kV_.alloc((size_t)(m + 1) * ld);
-    HY_CUDA(cudaMemsetAsync(kV_.p, 0, (size_t)(m + 1) * ld * sizeof(double), s));
-    std::vector<double> H((size_t)(m + 1) * m, 0.0), cs(m), sn(m), g(m + 1), hbuf(2 * m + 8);
-    double* dH1 = kH_.p;
-    double* dH2 = kH_.p + (m + 1);
-    double* dNrm = kH_.p + 2 * m + 2;
-    A(xc.p, kR_.p);
-    axpby(1.0, bc.p, -1.0, kR_.p, nOwn, s, &launches_);
-    const double r0norm = std::sqrt(dot(kR_.p, kR_.p));
-    double* r = kR_.p;
-    if (left) {
-      M(kR_.p, kZ_.p);
-      r = kZ_.p;
-    }
-    const double pr0norm = left ? std::sqrt(dot(r, r)) : r0norm;
-    auto scaleOf = [&](const std::string& k) {
-      double v = 1.0;
-      if (k == "Norm of RHS") v = bnorm;
-      else if (k == "Norm of Initial Residual") v = r0norm;
-      else if (k == "Norm of Preconditioned Initial Residual") v = pr0norm;
-      else if (k == "None") v = 1.0;
-      else throw Error(HYMLS_B200_ERR_ARG, "unknown residual scaling '" + k + "'");
-      return v == 0.0 ? 1.0 : v;
-    };
-    const double impScale = scaleOf(impScaling), expScale = scaleOf(expScaling);
-    double beta = pr0norm;
-    double trueRes = r0norm;
-    for (int restart = 0; restart <= maxRestarts; ++restart) {
-      if (restart == 0) history.push_back(beta / impScale);
-      lastRel = beta / impScale;
-      if (beta == 0.0 || (lastRel <= tol && !explicitTest)) {
-        converged = true;
-        break;
-      }
-      axpby(1.0 / beta, r, 0.0, kV_.p, nOwn, s, &launches_);
-      std::fill(g.begin(), g.end(), 0.0);
-      g[0] = beta;
-      int kDone = 0;
-      for (int k = 0; k < m && iters < maxIters; ++k) {
-        double* vk = kV_.p + (size_t)k * ld;
-        double* w = kV_.p + (size_t)(k + 1) * ld;
-        static const bool verboseSolve = getenv("HYMLS_B200_VERBOSE_SOLVE") != nullptr;
-        const bool lapIt = verboseSolve && comm_.rank() == 0 && (k % 50) == 20;
-        auto tl = std::chrono::steady_clock::now();
-        auto lapS = [&](const char* what) {
-          if (!lapIt) return;
-          cudaStreamSynchronize(s);
-          auto t1 = std::chrono::steady_clock::now();
-          fprintf(stderr, "[hymls_b200 solve dist] it %d %-28s %8.3f ms\n", k, what,
-                  std::chrono::duration<double, std::milli>(t1 - tl).count());
-          tl = t1;
-        };
-        if (lapIt) { cudaStreamSynchronize(s); tl = std::chrono::steady_clock::now(); }
-        if (right) {
-          Mglobal(vk, kX_.p);
-          lapS("ApplyInverse");
-          Aglobal(kX_.p, w);
-          lapS("matrix halo + spmv");
-        } else if (left) {
-          A(vk, kW_.p);
-          M(kW_.p, w);
-        } else {
-          A(vk, w);
-        }
-        multiDot(kV_.p, ld, k + 1, w, nOwn, kPartial_.p, dH1, 0, s, &launches_);
-        comm_.allReduceSum(dH1, (size_t)(k + 1), s);
-        multiAxpy(kV_.p, ld, k + 1, dH1, w, nOwn, -1.0, s, &launches_);
-        multiDot(kV_.p, ld, k + 1, w, nOwn, kPartial_.p, dH2, 0, s, &launches_);
-        comm_.allReduceSum(dH2, (size_t)(k + 1), s);
-        multiAxpy(kV_.p, ld, k + 1, dH2, w, nOwn, -1.0, s, &launches_);
-        multiDot(w, ld, 1, w, nOwn, kPartial_.p, dNrm, 0, s, &launches_);
-        comm_.allReduceSum(dNrm, 1, s);
-        scaleByInvNorm(w, dNrm, w, nOwn, s, &launches_);
-        lapS("CGS2 (4 sweeps, 3 allreduces)");
-        HY_CUDA(cudaMemcpyAsync(hbuf.data(), kH_.p, (2 * m + 3) * sizeof(double), cudaMemcpyDeviceToHost, s));
-        HY_CUDA(cudaStreamSynchronize(s));
-        lapS("Hessenberg column to host");
-        for (int i = 0; i <= k; ++i) H[(size_t)i * m + k] = hbuf[i] + hbuf[m + 1 + i];
-        const double hn = std::sqrt(hbuf[2 * m + 2]);
-        double colNorm = 0.0;
-        for (int i = 0; i <= k; ++i) colNorm = std::hypot(colNorm, hbuf[i] + hbuf[m + 1 + i]);
-        const bool breakdown = !(hn > 1e-300) || hn <= 1e-15 * colNorm;
-        H[(size_t)(k + 1) * m + k] = breakdown ? 0.0 : hn;
-        for (int i = 0; i < k; ++i) {
-          const double t = cs[i] * H[(size_t)i * m + k] + sn[i] * H[(size_t)(i + 1) * m + k];
-          H[(size_t)(i + 1) * m + k] = -sn[i] * H[(size_t)i * m + k] + cs[i] * H[(size_t)(i + 1) * m + k];
-          H[(size_t)i * m + k] = t;
-        }
-        const double d = std::hypot(H[(size_t)k * m + k], H[(size_t)(k + 1) * m + k]);
-        cs[k] = H[(size_t)k * m + k] / d;
-        sn[k] = H[(size_t)(k + 1) * m + k] / d;
-        H[(size_t)k * m + k] = d;
-        H[(size_t)(k + 1) * m + k] = 0.0;
-        g[k + 1] = -sn[k] * g[k];
-        g[k] = cs[k] * g[k];
-        ++iters;
-        kDone = k + 1;
-        lastRel = std::fabs(g[k + 1]) / impScale;
-        history.push_back(lastRel);
-        if (lastRel <= tol || breakdown) break;
-      }
-      if (kDone > 0) {
-        std::vector<double> y(kDone);
-        for (int i = kDone - 1; i >= 0; --i) {
-          double t = g[i];
-          for (int j = i + 1; j < kDone; ++j) t -= H[(size_t)i * m + j] * y[j];
-          y[i] = t / H[(size_t)i * m + i];
-        }
-        HY_CUDA(cudaMemcpyAsync(dH1, y.data(), kDone * sizeof(double), cudaMemcpyHostToDevice, s));
-        HY_CUDA(cudaMemsetAsync(kW_.p, 0, ld * sizeof(double), s));
-        multiAxpy(kV_.p, ld, kDone, dH1, kW_.p, nOwn, 1.0, s, &launches_);
-        HY_CUDA(cudaStreamSynchronize(s));
-        if (right) {
-          M(kW_.p, kZ_.p);
-          axpby(1.0, kZ_.p, 1.0, xc.p, nOwn, s, &launches_);
-        } else {
-          axpby(1.0, kW_.p, 1.0, xc.p, nOwn, s, &launches_);
-        }
-      }
-      A(xc.p, kR_.p);
-      axpby(1.0, bc.p, -1.0, kR_.p, nOwn, s, &launches_);
-      trueRes = std::sqrt(dot(kR_.p, kR_.p));
-      r = kR_.p;
-      beta = trueRes;
-      if (left) {
-        M(kR_.p, kZ_.p);
-        r = kZ_.p;
-        beta = std::sqrt(dot(r, r));
-      }
-      if (history.back() <= tol) {
-        if (!explicitTest || trueRes / expScale <= tol) {
-          converged = true;
-          break;
-        }
-      }
-      if (iters >= maxIters) break;
-    }
-  } else {
-    throw Error(HYMLS_B200_ERR_ARG, "Krylov Method '" + method + "' not supported (GMRES, CG)");
-  }
-  HY_CUDA(cudaEventRecord(ev1_, s));
-  HY_CUDA(cudaStreamSynchronize(s));
-  float ms = 0;
-  HY_CUDA(cudaEventElapsedTime(&ms, ev0_, ev1_));
-  A(xc.p, kR_.p);
-  axpby(1.0, bc.p, -1.0, kR_.p, nOwn, s, &launches_);
-  const double res = std::sqrt(dot(kR_.p, kR_.p));
-  // replicated result, like the single-GPU entry point
-  toGlobal(xc.p, kB_.p);
-  gatherOwned(kB_.p, kX_.p);
-  const auto back = where == HYMLS_B200_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-  HY_CUDA(cudaMemcpyAsync(x, kX_.p, n * sizeof(double), back, s));
-  HY_CUDA(cudaStreamSynchronize(s));
-  if (info) {
-    info->iterations = iters;
-    info->converged = converged ? 1 : 0;
-    info->rel_residual = lastRel;
-    info->explicit_rel_residual = bnorm > 0 ? res / bnorm : res;
-    info->solve_seconds = ms * 1e-3;
-    info->history_len = (int)history.size();
-  }
-  if (hist)
-    for (int i = 0; i < (int)history.size() && i < histCap; ++i) hist[i] = history[i];
 }
 
 }  // namespace hymls

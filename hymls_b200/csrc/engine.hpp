@@ -157,6 +157,8 @@ struct DistMatrixCache {
 };
 
 // block-tridiagonal coarse factorization on BFS level sets (coarse.cu)
+struct KrylovLayout;  // the vector layout of one Krylov solve (krylov.cu)
+
 struct CoarseBT {
   bool planned = false, active = false;
   int n = 0, m = 0;
@@ -241,8 +243,9 @@ class Engine {
   void haloExchange(Halo& h, const double* src, double* dst, bool scatter);
   void applyLevel0Dist(const double* B, double* X);
   void gatherOwned(const double* Xowned, double* Xfull);
-  void solveDist(const double* b, double* x, int where, uint64_t seed, hymls_b200_solve_info* info, double* hist,
-                 int histCap);
+  // Krylov solves on replicated vectors and on the owner distribution (krylov.cu)
+  KrylovLayout replicatedLayout(bool left, bool right);
+  KrylovLayout ownerLayout(bool left, bool right);
   void applyDevice(const double* dB, double* dX, const double* dT = nullptr, double* dS = nullptr);
   bool applyDeviceMulti(const double* dB, int64_t ldb, double* dX, int64_t ldx, int nv);
   DevBuf<double> x1m_, y1m_;  // interior work vectors of the multi-column apply
@@ -283,7 +286,8 @@ class Engine {
   DevBuf<double> bufG_;          // compact staging of the distributed-vector entry point
   DevBuf<double> bufD_;          // global-length scratch of the owner-computes path
   // Krylov workspace
-  DevBuf<double> kV_, kW_, kZ_, kH_, kPartial_, kX_, kB_, kR_;
+  DevBuf<double> kV_, kW_, kZ_, kH_, kPartial_, kX_, kB_, kR_, kQ_;
+  DevBuf<double> kS1_, kS2_;  // scratch of the vector layouts
   int kCap_ = 0;
   // statistics
   hymls_b200_stats stats_{};
