@@ -37,7 +37,8 @@ class _Stats(C.Structure):
                 ("bytes_apply", C.c_double), ("flops_compute", C.c_double), ("bytes_a11_level0", C.c_double),
                 ("kernel_launches", C.c_int64), ("device_bytes", C.c_double), ("sum_nsd_nb", C.c_double),
                 ("bytes_a11_full_pass", C.c_double), ("ms_a11_lead", C.c_double), ("interior_couplings", C.c_int64),
-                ("a11_split", C.c_int64), ("host_pipeline_chunks", C.c_int64), ("host_pipeline_state", C.c_int64)]
+                ("a11_split", C.c_int64), ("host_pipeline_chunks", C.c_int64), ("host_pipeline_state", C.c_int64),
+                ("collective_calls", C.c_int64), ("collective_bytes", C.c_int64)]
 
 
 def lib_path():
@@ -82,6 +83,9 @@ def load_library():
     lib.hymls_b200_owned_rows.argtypes = [vp, vp, i64]
     lib.hymls_b200_owned_rows.restype = i64
     lib.hymls_b200_apply_inverse_dist.argtypes = [vp, vp, vp, C.c_int]
+    lib.hymls_b200_apply_inverse_bordered_dist.argtypes = [vp, vp, vp, vp, vp, C.c_int]
+    lib.hymls_b200_border_size.argtypes = [vp]
+    lib.hymls_b200_get_device.argtypes = [vp]
     lib.hymls_b200_set_border.argtypes = [vp, vp, vp, vp, C.c_int]
     lib.hymls_b200_apply_inverse_bordered.argtypes = [vp, vp, i64, vp, vp, i64, vp, C.c_int, C.c_int]
     lib.hymls_b200_apply_matrix.argtypes = [vp, vp, vp, C.c_int]
@@ -338,6 +342,10 @@ class Preconditioner:
             self._h, Vc.ctypes.data, None if Wc is None else Wc.ctypes.data,
             None if Cc is None else Cc.ctypes.data, m))
 
+    def BorderSize(self):
+        """m of the border set with SetBorder or hymls_b200_set_border_dist (0: none)"""
+        return self._lib.hymls_b200_border_size(self._h)
+
     def ApplyInverseBordered(self, B, T):
         """[X; S] = [K V; W' C]^-1 [B; T] approximately (BorderedOperator::ApplyInverse of the preconditioner,
         src/HYMLS_Preconditioner.cpp:930-1070).  numpy, host: B is n (x nvec), T is m (x nvec)."""
@@ -349,6 +357,48 @@ class Preconditioner:
         _check(self._lib, self._lib.hymls_b200_apply_inverse_bordered(
             self._h, Bc.ctypes.data, self.n, Tc.ctypes.data, Xc.ctypes.data, self.n, Sc.ctypes.data, nvec, HOST))
         return Xc, Sc
+
+    def ApplyInverseBorderedDist(self, b_local, T):
+        """[x; S] = [K V; W' C]^-1 [b; T] on the rows of OwnedRows(): b_local holds those rows, T (length m, the same on
+        every rank) the border right-hand side; returns (x_local, S), S bitwise equal on every rank.  Both numpy
+        (host buffers) or both 1-D torch CUDA tensors on the handle's device (device buffers), float64 and
+        contiguous."""
+        m = self.BorderSize()
+        if m == 0:
+            raise ValueError("ApplyInverseBorderedDist: no border set (SetBorder)")
+        nown = int(self._lib.hymls_b200_owned_rows(self._h, None, 0))
+        _check(self._lib, nown)
+
+        def need(ok, what):
+            if not ok:
+                raise ValueError("ApplyInverseBorderedDist: " + what)
+
+        if isinstance(b_local, np.ndarray):
+            need(isinstance(T, np.ndarray), "b_local is a numpy array, so T must be one")
+            for name, a, ln in (("b_local", b_local, nown), ("T", T, m)):
+                need(a.dtype == np.float64, "%s must be float64" % name)
+                need(a.ndim == 1 and a.shape[0] == ln, "%s must be 1-D of length %d" % (name, ln))
+                need(a.flags.c_contiguous, "%s must be contiguous" % name)
+            xl = np.zeros(nown)
+            S = np.zeros(m)
+            where = HOST
+        else:
+            import torch
+            need(isinstance(b_local, torch.Tensor) and isinstance(T, torch.Tensor), "expected numpy arrays or torch tensors")
+            dev = _check(self._lib, self._lib.hymls_b200_get_device(self._h))
+            for name, a, ln in (("b_local", b_local, nown), ("T", T, m)):
+                need(a.is_cuda and a.device.index == dev, "%s must be a CUDA tensor on cuda:%d, the handle's device"
+                     % (name, dev))
+                need(a.dtype == torch.float64, "%s must be float64" % name)
+                need(a.dim() == 1 and a.shape[0] == ln, "%s must be 1-D of length %d" % (name, ln))
+                need(a.is_contiguous(), "%s must be contiguous" % name)
+            xl = torch.empty_like(b_local)
+            S = torch.empty_like(T)
+            where = DEVICE
+        p = lambda a: a.ctypes.data if where == HOST else a.data_ptr()  # noqa: E731
+        _check(self._lib, self._lib.hymls_b200_apply_inverse_bordered_dist(self._h, p(b_local), p(T), p(xl), p(S),
+                                                                            where))
+        return xl, S
 
     def ApplyMatrix(self, x):
         if isinstance(x, np.ndarray):

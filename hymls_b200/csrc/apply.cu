@@ -409,13 +409,14 @@ void householder(const int* uniqStart, int nuniq, const double* w, const double*
 // ---------------------------------------------------------------------------------------------
 // small vector kernels of the Krylov loop
 // ---------------------------------------------------------------------------------------------
-// partial[i * nblk + b] = sum over rows of block b of V_i[r] * w[r],  i = 0..k-1.
+// partial[i * nblk + b] = sum over rows of block b of V_i[r] * w[r],  i = 0..k-1; r runs over [0, n) or, with a row
+// list, over rows[0..n).
 // The basis vectors are taken DOT_G at a time: one read of w[r] feeds DOT_G products with independent loads
 // in flight, and the block reduction is paid once per group instead of once per vector.
 static constexpr int DOT_G = 8;
 __global__ void __launch_bounds__(256)
 k_multi_dot(const double* __restrict__ V, int64_t ldv, int k, const double* __restrict__ w, int64_t n,
-            double* __restrict__ partial, const int* __restrict__ widx) {
+            double* __restrict__ partial, const int* __restrict__ widx, const int* __restrict__ rows) {
   __shared__ double red[DOT_G][8];
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -426,13 +427,15 @@ k_multi_dot(const double* __restrict__ V, int64_t ldv, int k, const double* __re
 #pragma unroll
     for (int g = 0; g < DOT_G; ++g) acc[g] = 0.0;
     if (ng == DOT_G) {
-      for (int64_t r = (int64_t)blockIdx.x * blockDim.x + tid; r < n; r += stride) {
+      for (int64_t i = (int64_t)blockIdx.x * blockDim.x + tid; i < n; i += stride) {
+        const int64_t r = rows ? (int64_t)rows[i] : i;
         const double wv = widx ? w[widx[r]] : w[r];
 #pragma unroll
         for (int g = 0; g < DOT_G; ++g) acc[g] += v0[(int64_t)g * ldv + r] * wv;
       }
     } else {
-      for (int64_t r = (int64_t)blockIdx.x * blockDim.x + tid; r < n; r += stride) {
+      for (int64_t i = (int64_t)blockIdx.x * blockDim.x + tid; i < n; i += stride) {
+        const int64_t r = rows ? (int64_t)rows[i] : i;
         const double wv = widx ? w[widx[r]] : w[r];
 #pragma unroll
         for (int g = 0; g < DOT_G; ++g)
@@ -479,9 +482,9 @@ __global__ void k_reduce_partials(const double* __restrict__ partial, int nblk, 
 }
 static const int DOT_BLOCKS = 592;  // 4 x 148 SMs
 void multiDot(const double* V, int64_t ldv, int k, const double* w, int64_t n, double* partial, double* h,
-              int accumulate, cudaStream_t s, int64_t* launches, const int* widx) {
+              int accumulate, cudaStream_t s, int64_t* launches, const int* widx, const int* rows) {
   if (k == 0) return;
-  k_multi_dot<<<DOT_BLOCKS, 256, 0, s>>>(V, ldv, k, w, n, partial, widx);
+  k_multi_dot<<<DOT_BLOCKS, 256, 0, s>>>(V, ldv, k, w, n, partial, widx, rows);
   k_reduce_partials<<<k, 256, 0, s>>>(partial, DOT_BLOCKS, k, h, accumulate);
   *launches += 2;
 }
@@ -813,18 +816,21 @@ void zeroAt(double* x, const int* idx, int64_t n, cudaStream_t s, int64_t* launc
   ++*launches;
 }
 // X[idx[p]] -= sum_j Q[j*ld + p] * S[j]    (x1 -= Q1 S of the bordered ApplyInverse, Preconditioner.cpp:1036-1041)
+// for p in [0, n) or, with a position list, p = list[0..n)
 __global__ void k_border_correct(double* __restrict__ X, const int* __restrict__ idx, const double* __restrict__ Q,
-                                 int64_t ld, int m, const double* __restrict__ S, int64_t n) {
-  const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= n) return;
+                                 int64_t ld, int m, const double* __restrict__ S, int64_t n,
+                                 const int* __restrict__ list) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int64_t p = list ? (int64_t)list[i] : i;
   double t = 0.0;
   for (int j = 0; j < m; ++j) t += Q[(int64_t)j * ld + p] * S[j];
   X[idx[p]] -= t;
 }
 void borderCorrect(double* X, const int* idx, const double* Q, int64_t ld, int m, const double* S, int64_t n,
-                   cudaStream_t s, int64_t* launches) {
+                   cudaStream_t s, int64_t* launches, const int* list) {
   if (n == 0 || m == 0) return;
-  k_border_correct<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(X, idx, Q, ld, m, S, n);
+  k_border_correct<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(X, idx, Q, ld, m, S, n, list);
   ++*launches;
 }
 // augmented dense matrix [D V; W' C]: D is n x n inside an np x np row-major array, V, W are n x m
@@ -847,6 +853,65 @@ void denseBorder(double* D, int n, int np, const double* V, const double* W, int
   if (m == 0) return;
   k_dense_border<<<(n + m + 255) / 256, 256, 0, s>>>(D, n, np, V, W, ld, C, m);
   ++*launches;
+}
+
+// Rows r = rows[i] of the bordered operator [K V; W' C] on the owner distribution, one pass over the owned rows:
+//   y[i] = sum_e val[e] x[col[e]] + sum_j V[j*ld + r] sv[j]
+//   partial[j * gridDim.x + b] = sum over the rows of block b of W[j*ld + r] x[r]    (reduced like multiDot)
+// x is a global-length vector valid at the owned rows and their matrix halo, sv the border part of the argument.
+static constexpr int BORDER_G = 8;  // border columns per sweep of the dot part (m > 8 re-reads x)
+__global__ void __launch_bounds__(256)
+k_border_spmv_rows(const int64_t* __restrict__ ptr, const int* __restrict__ col, const double* __restrict__ val,
+                   const double* __restrict__ x, const double* __restrict__ V, const double* __restrict__ W, int64_t ld,
+                   int m, const double* __restrict__ sv, const int* __restrict__ rows, int64_t nrows,
+                   double* __restrict__ y, double* __restrict__ partial) {
+  __shared__ double red[BORDER_G][8];
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int j0 = 0; j0 < m; j0 += BORDER_G) {
+    const int ng = min(BORDER_G, m - j0);
+    double acc[BORDER_G];
+#pragma unroll
+    for (int g = 0; g < BORDER_G; ++g) acc[g] = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + tid; i < nrows; i += stride) {
+      const int64_t r = rows[i];
+      const double xr = x[r];
+      if (j0 == 0) {
+        double s = 0.0;
+        for (int64_t e = ptr[r]; e < ptr[r + 1]; ++e) s += val[e] * x[col[e]];
+        double t = 0.0;
+        for (int j = 0; j < m; ++j) t += V[(int64_t)j * ld + r] * sv[j];
+        y[i] = s + t;
+      }
+#pragma unroll
+      for (int g = 0; g < BORDER_G; ++g)
+        if (g < ng) acc[g] += W[(int64_t)(j0 + g) * ld + r] * xr;
+    }
+#pragma unroll
+    for (int g = 0; g < BORDER_G; ++g) {
+      double s = acc[g];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+      if (lane == 0) red[g][wid] = s;
+    }
+    __syncthreads();
+    if (tid < BORDER_G * 8) {
+      const int g = tid >> 3, j = tid & 7;
+      double s = red[g][j];
+#pragma unroll
+      for (int o = 4; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o, 8);
+      if (j == 0 && g < ng) partial[(int64_t)(j0 + g) * gridDim.x + blockIdx.x] = s;
+    }
+    __syncthreads();
+  }
+}
+void borderSpmvRows(const int64_t* ptr, const int* col, const double* val, const double* x, const double* V,
+                    const double* W, int64_t ld, int m, const double* sv, const int* rows, int64_t nrows, double* y,
+                    double* partial, double* dots, cudaStream_t s, int64_t* launches) {
+  if (m == 0) return;
+  k_border_spmv_rows<<<DOT_BLOCKS, 256, 0, s>>>(ptr, col, val, x, V, W, ld, m, sv, rows, nrows, y, partial);
+  k_reduce_partials<<<m, 256, 0, s>>>(partial, DOT_BLOCKS, m, dots, 0);
+  *launches += 2;
 }
 
 // out[i - i0] = dots[i] + sum_j C[i + j*m] sv[j]  (border rows of BorderedOperator::Apply)

@@ -211,6 +211,24 @@ int hymls_b200_apply_inverse_dist(hymls_b200_t* h, const double* Bl, double* Xl,
   HY_CATCH
 }
 
+int hymls_b200_apply_inverse_bordered_dist(hymls_b200_t* h, const double* Bl, const double* T, double* Xl, double* S,
+                                           int where) {
+  HY_TRY
+  if (!T || !S) throw Error(HYMLS_B200_ERR_ARG, "apply_inverse_bordered_dist: T and S are required");
+  h->eng->applyInverseDist(Bl, Xl, where, T, S);
+  return 0;
+  HY_CATCH
+}
+
+int hymls_b200_border_size(hymls_b200_t* h) { return h->eng->borderSize(); }
+
+int hymls_b200_get_device(hymls_b200_t* h) {
+  HY_TRY
+  if (h->eng->device() < 0) throw Error(HYMLS_B200_ERR_CUDA, "no CUDA device");
+  return h->eng->device();
+  HY_CATCH
+}
+
 int hymls_b200_set_border(hymls_b200_t* h, const double* V, const double* W, const double* C, int m) {
   HY_TRY
   h->eng->setBorder(V, W, C, m);

@@ -118,6 +118,7 @@ void Comm::allReduceSum(double* buf, size_t count, cudaStream_t s) const {
   const int ncclDouble = 8, ncclSum = 0;  // ncclFloat64, ncclSum (nccl.h enums, stable across 2.x)
   static const bool syncEach = getenv("HYMLS_B200_SYNC_NCCL") != nullptr;
   if (syncEach) cudaStreamSynchronize(s);
+  tally(count);
   check(api().allReduce(buf, buf, count, ncclDouble, ncclSum, comm_, s), "ncclAllReduce");
   if (syncEach) cudaStreamSynchronize(s);
 }
@@ -128,11 +129,13 @@ namespace hymls {
 void Comm::allGather(const double* send, double* recv, size_t count, cudaStream_t s) const {
   if (!comm_ || count == 0) return;
   const int ncclDouble = 8;
+  tally(count);
   check(api().allGather(send, recv, count, ncclDouble, comm_, s), "ncclAllGather");
 }
 void Comm::broadcast(double* buf, size_t count, int root, cudaStream_t s) const {
   if (!comm_ || count == 0) return;
   const int ncclDouble = 8;
+  tally(count);
   check(api().broadcast(buf, buf, count, ncclDouble, root, comm_, s), "ncclBroadcast");
 }
 }  // namespace hymls
@@ -152,6 +155,10 @@ void Comm::neighbourExchange(const std::vector<int>& peers, const double* sendBu
   }
   if (!comm_ || !others) return;
   const int ncclDouble = 8;
+  size_t moved = 0;
+  for (size_t k = 0; k < peers.size(); ++k)
+    if (peers[k] != rank_) moved += (size_t)(sendPtr[k + 1] - sendPtr[k] + recvPtr[k + 1] - recvPtr[k]);
+  tally(moved);
   Api& a = api();
   check(a.groupStart(), "ncclGroupStart");
   for (size_t k = 0; k < peers.size(); ++k) {

@@ -28,10 +28,16 @@ class Comm {
   // grouped ncclSend / ncclRecv with a set of neighbour ranks (halo exchange)
   void neighbourExchange(const std::vector<int>& peers, const double* sendBuf, const std::vector<int64_t>& sendPtr,
                          double* recvBuf, const std::vector<int64_t>& recvPtr, cudaStream_t s) const;
+  // this rank's collective calls and their payload bytes since init (all-reduce / broadcast / all-gather: the count
+  // of one rank; neighbour exchange: sent + received to / from other ranks).  The warm-up of init is not counted.
+  int64_t calls() const { return calls_; }
+  int64_t bytes() const { return bytes_; }
 
  private:
   void* comm_ = nullptr;
   int rank_ = 0, nranks_ = 1;
+  mutable int64_t calls_ = 0, bytes_ = 0;
+  void tally(size_t doubles) const { calls_++; bytes_ += (int64_t)(doubles * sizeof(double)); }
 };
 
 }  // namespace hymls

@@ -51,6 +51,7 @@ Engine::Engine(const std::string& xml) {
   if (!deviceOk_) cudaGetLastError();
   readParameters();
   if (deviceOk_) {
+    HY_CUDA(cudaGetDevice(&device_));
     HY_CUDA(cudaEventCreate(&ev0_));
     HY_CUDA(cudaEventCreate(&ev1_));
     HY_CUDA(cudaEventCreate(&evA_));
@@ -1830,16 +1831,15 @@ bool Engine::applyDeviceMulti(const double* dB, int64_t ldb, double* dX, int64_t
 }
 
 void Engine::applyDevice(const double* dB, double* dX, const double* dT, double* dS) {
-  if (useDist() && !dT) {
+  if (useDist()) {
     // replicated argument / result around the owner-computes path: every rank applies to its own rows, the
-    // owned parts of the result are all-gathered
+    // owned parts of the result are all-gathered (S is replicated already)
     bufD_.alloc(n_);
-    applyLevel0Dist(dB, bufD_.p);
+    applyLevel0Dist(dB, bufD_.p, dT);
     gatherOwned(bufD_.p, dX);
-    stats_.num_apply_inverse++;
-    return;
+  } else {
+    applyLevel(0, dB, dX, dT);
   }
-  applyLevel(0, dB, dX, dT);
   if (dS && borderM_)
     HY_CUDA(cudaMemcpyAsync(dS, bS_.p, borderM_ * sizeof(double), cudaMemcpyDeviceToDevice, stream_));
   stats_.num_apply_inverse++;
@@ -2057,13 +2057,16 @@ void Engine::localRows(int64_t* r0, int64_t* r1) const {
 }
 
 // Distributed-vector ApplyInverse: Bloc / Xloc hold the rows hymls_b200_owned_rows lists (ascending), i.e. the
-// distribution the subdomain -> rank map of the reference induces
-void Engine::applyInverseDist(const double* Bloc, double* Xloc, int where) {
+// distribution the subdomain -> rank map of the reference induces.  With T and S (replicated m-vectors, on the same
+// side as Bloc) it is the bordered ApplyInverse; without them and a border set, T = 0 and S is discarded.
+void Engine::applyInverseDist(const double* Bloc, double* Xloc, int where, const double* T, double* S) {
   needDevice();
   needComm();
   if (!computed_) throw Error(HYMLS_B200_ERR_STATE, "The preconditioner has not yet been computed.");
+  const int bm = T ? borderM_ : 0;  // no border set: m = 0, S has no entries and is not written
   if (comm_.size() <= 1) {
-    applyInverse(Bloc, n_, Xloc, n_, 1, where);
+    if (bm) applyInverseBordered(Bloc, n_, T, Xloc, n_, S, 1, where);
+    else applyInverse(Bloc, n_, Xloc, n_, 1, where);
     return;
   }
   DistPlan& D = levels_[0]->dist;
@@ -2079,9 +2082,11 @@ void Engine::applyInverseDist(const double* Bloc, double* Xloc, int where) {
   const auto out = where == HYMLS_B200_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
   HY_CUDA(cudaMemcpyAsync(cB, Bloc, D.nOwn * sizeof(double), in, s));
   scatterVec(cB, D.ownRows.p, bufB_.p, D.nOwn, s, &launches_);
-  applyOwned(bufB_.p, bufX_.p);
+  if (bm) HY_CUDA(cudaMemcpyAsync(bTin_.p, T, bm * sizeof(double), in, s));
+  applyOwned(bufB_.p, bufX_.p, bm ? bTin_.p : nullptr);
   packIdx(bufX_.p, D.ownRows.p, cX, D.nOwn, s, &launches_);
   HY_CUDA(cudaMemcpyAsync(Xloc, cX, D.nOwn * sizeof(double), out, s));
+  if (bm) HY_CUDA(cudaMemcpyAsync(S, bS_.p, bm * sizeof(double), out, s));
   if (where == HYMLS_B200_HOST) HY_CUDA(cudaStreamSynchronize(s));
 }
 
@@ -2090,9 +2095,9 @@ void Engine::applyOwned(const double* Bglobal, double* Xglobal, const double* dT
     applyDevice(Bglobal, Xglobal, dT, nullptr);  // (S stays in bS_)
     return;
   }
-  if (useDist() && !dT) {
-    applyLevel0Dist(Bglobal, Xglobal);
-  } else {  // bordered / fallback path works on replicated vectors
+  if (useDist()) {
+    applyLevel0Dist(Bglobal, Xglobal, dT);
+  } else {  // fallback path (HYMLS_B200_DIST=0, Number of Levels = 0) works on replicated vectors
     bufD_.alloc(n_);
     gatherOwned(Bglobal, bufD_.p);
     applyLevel(0, bufD_.p, Xglobal, dT);
@@ -2267,6 +2272,8 @@ void Engine::getStats(hymls_b200_stats* st) {
     }
     st->bytes_apply = bytes;
   }
+  st->collective_calls = comm_.calls();
+  st->collective_bytes = comm_.bytes();
 }
 
 }  // namespace hymls

@@ -195,9 +195,10 @@ class Engine {
   void applyInverseBordered(const double* B, int64_t ldb, const double* T, double* X, int64_t ldx, double* S, int nvec,
                             int where);
   int borderSize() const { return borderM_; }
+  int device() const { return device_; }  // CUDA device the handle is bound to (-1: none)
   void applyMatrix(const double* x, double* y, int where);
   void localRows(int64_t* r0, int64_t* r1) const;
-  void applyInverseDist(const double* Bloc, double* Xloc, int where);
+  void applyInverseDist(const double* Bloc, double* Xloc, int where, const double* T = nullptr, double* S = nullptr);
   int64_t ownedRows(int64_t* rows, int64_t cap);
   void solve(const double* b, double* x, int where, uint64_t seed, hymls_b200_solve_info* info, double* hist,
              int histCap);
@@ -241,7 +242,7 @@ class Engine {
   void buildDistPlan(Level& L);
   void buildMatrixHalo();
   void haloExchange(Halo& h, const double* src, double* dst, bool scatter);
-  void applyLevel0Dist(const double* B, double* X);
+  void applyLevel0Dist(const double* B, double* X, const double* T = nullptr);  // with a border: S -> bS_
   void gatherOwned(const double* Xowned, double* Xfull);
   // Krylov solves on replicated vectors and on the owner distribution (krylov.cu)
   KrylovLayout replicatedLayout(bool left, bool right);
@@ -261,6 +262,7 @@ class Engine {
   std::vector<int> hColidx_;
   std::vector<double> hTestVector_;
   bool haveMatrix_ = false, initialized_ = false, computed_ = false, deviceOk_ = false;
+  int device_ = -1;
   void needDevice() const;
   void needComm() const;
   std::vector<std::unique_ptr<Level>> levels_;

@@ -163,8 +163,10 @@ void scatterValues(const double* src, const int64_t* srcIdx, const int64_t* dstI
                    int64_t n, cudaStream_t s, int64_t* launches);
 void householder(const int* uniqStart, int nuniq, const double* w, const double* in, double* out, double* vsumOut,
                  const double* vsumIn, double* X, const int* sepRow, cudaStream_t s, int64_t* launches);
+// h[i] (+)= V_i' w over the rows r in [0, n), or r = rows[0..n) with a row list; widx: w[widx[r]].  Deterministic
+// (fixed reduction order, no atomics).
 void multiDot(const double* V, int64_t ldv, int k, const double* w, int64_t n, double* partial, double* h,
-              int accumulate, cudaStream_t s, int64_t* launches, const int* widx = nullptr);  // widx: w[widx[r]]
+              int accumulate, cudaStream_t s, int64_t* launches, const int* widx = nullptr, const int* rows = nullptr);
 int multiDotBlocks();
 
 void multiAxpy(const double* V, int64_t ldv, int k, const double* h, double* w, int64_t n, double sign,
@@ -203,12 +205,18 @@ void batchedGemvT(const GemvArgs& a, int count, int npMax, cudaStream_t s, int64
 void spmvIndexed(const int64_t* ptr, const int* col, const int64_t* idx, const double* val, const double* x, double* y,
                  int64_t n, double alpha, cudaStream_t s, int64_t* launches);
 void zeroAt(double* x, const int* idx, int64_t n, cudaStream_t s, int64_t* launches);
+// X[idx[p]] -= sum_j Q[j*ld + p] S[j] for p in [0, n), or p = list[0..n) with a position list
 void borderCorrect(double* X, const int* idx, const double* Q, int64_t ld, int m, const double* S, int64_t n,
-                   cudaStream_t s, int64_t* launches);
+                   cudaStream_t s, int64_t* launches, const int* list = nullptr);
 void denseBorder(double* D, int n, int np, const double* V, const double* W, int64_t ld, const double* C, int m,
                  cudaStream_t s, int64_t* launches);
 
 void borderRows(const double* dots, const double* C, const double* sv, int m, int i0, int i1, double* out,
                 cudaStream_t s, int64_t* launches);
+// owned rows r = rows[i] of [K V; W' C] in one pass: y[i] = (K x)[r] + (V sv)[r], dots[j] = sum_i W[j*ld + r] x[r]
+// (this rank's partial sums, deterministic; partial: m * multiDotBlocks() doubles)
+void borderSpmvRows(const int64_t* ptr, const int* col, const double* val, const double* x, const double* V,
+                    const double* W, int64_t ld, int m, const double* sv, const int* rows, int64_t nrows, double* y,
+                    double* partial, double* dots, cudaStream_t s, int64_t* launches);
 
 }  // namespace hymls

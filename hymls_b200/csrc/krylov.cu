@@ -2,9 +2,10 @@
 //
 // One GMRES(m) / CG serves both vector layouts of the library; KrylovLayout carries the operations in which they
 // differ:
-//   * replicated: every rank holds whole vectors of length n (+ border).  One GPU, bordered systems, and several
-//     ranks without the owner path (HYMLS_B200_DIST=0, Number of Levels = 0, a border).
-//   * owner: a rank holds the rows it owns (DistPlan, dist.cu), packed; useDist() selects it.
+//   * replicated: every rank holds whole vectors of length n (+ border).  One GPU, and several ranks without the
+//     owner path (HYMLS_B200_DIST=0, Number of Levels = 0).
+//   * owner: a rank holds the rows it owns (DistPlan, dist.cu), packed, followed by the border entries, which every
+//     rank keeps (bitwise equal); useDist() selects it.
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -16,10 +17,11 @@
 namespace hymls {
 
 // Solution-side vectors are what the driver keeps x, b, r, z in: `len` entries on this rank, `ld` allocated.  Every
-// rank stores rows [row0, row0 + rows) of them in the GMRES basis, with stride rowLd.
+// rank stores rows [row0, row0 + rows) of them in the GMRES basis, with stride rowLd; the first dotRows of those
+// rows enter this rank's partial sums of the inner products (rows stored on several ranks are counted on one).
 struct KrylovLayout {
   int64_t len = 0, ld = 0;
-  int64_t rows = 0, rowLd = 0, row0 = 0;
+  int64_t rows = 0, rowLd = 0, row0 = 0, dotRows = 0;
   std::function<void(const double* in, double* out)> A, M;  // operator, preconditioner on solution-side vectors
   std::function<void(const double* u, const double* v, double* d)> dot;  // *d = u'v on the device
   // the Arnoldi step w = A M^-1 v, M^-1 A v or A v on basis rows; it may use kZ_ and kW_, which the driver leaves
@@ -56,7 +58,7 @@ KrylovLayout Engine::replicatedLayout(bool left, bool right) {
   }
   KrylovLayout L;
   L.len = L.ld = n;
-  L.rows = nloc;
+  L.rows = L.dotRows = nloc;
   L.rowLd = chunk;
   L.row0 = r0;
   auto A = [=](const double* in, double* out) { operatorRows(in, out, 0, n); };
@@ -104,52 +106,65 @@ KrylovLayout Engine::replicatedLayout(bool left, bool right) {
   return L;
 }
 
-// Packed owned rows; the basis lives in the same rows, so the loop contains no full-vector collective.  The operator
-// and the preconditioner work on global-length vectors with the owned entries valid: kS1_ (argument) and kS2_
-// (result).
+// Packed owned rows, then the m border entries (bordered system [K V; W' C], replicated: only rank 0 counts them in
+// the inner products); the basis lives in the same rows, so the loop contains no full-vector collective.  The
+// operator and the preconditioner work on global-length vectors with the owned entries valid: kS1_ (argument) and
+// kS2_ (result); the border adds one all-reduce of m doubles to the operator.
 KrylovLayout Engine::ownerLayout(bool left, bool right) {
   Level* L0 = levels_[0].get();
   DistPlan* D = &L0->dist;
   buildMatrixHalo();
   cudaStream_t s = stream_;
-  const int64_t n = n_, nOwn = D->nOwn, ld = (D->maxOwn + 7) & ~(int64_t)7;
+  const int bm = borderM_;
+  const int64_t n = n_, nOwn = D->nOwn, ld = (D->maxOwn + bm + 7) & ~(int64_t)7;
   kS1_.alloc(n);
   kS2_.alloc(n);
   double* gIn = kS1_.p;
   double* gOut = kS2_.p;
   KrylovLayout L;
-  L.len = L.rows = nOwn;
+  L.len = L.rows = nOwn + bm;
+  L.dotRows = nOwn + (comm_.rank() == 0 ? bm : 0);
   L.ld = L.rowLd = ld;
   L.row0 = 0;
+  const int64_t dotRows = L.dotRows;
   auto toGlobal = [=](const double* c, double* full) { scatterVec(c, D->ownRows.p, full, nOwn, s, &launches_); };
-  auto Aglobal = [=](double* full, double* outC) {  // halo of `full` is filled in place
+  // outC = [K V; W' C] [full; sv] on the owned rows + the border rows; the halo of `full` is filled in place
+  auto Aglobal = [=](double* full, const double* sv, double* outC) {
     haloExchange(D->mat, full, full, true);
-    spmvRows(L0->rowptr.p, L0->colidx.p, L0->val.p, full, outC, D->ownRows.p, nOwn, 0.0, nullptr, nullptr, 1.0, 1, s,
-             &launches_);
+    if (!bm) {
+      spmvRows(L0->rowptr.p, L0->colidx.p, L0->val.p, full, outC, D->ownRows.p, nOwn, 0.0, nullptr, nullptr, 1.0, 1, s,
+               &launches_);
+      return;
+    }
+    borderSpmvRows(L0->rowptr.p, L0->colidx.p, L0->val.p, full, L0->bV.p, L0->bW.p, n, bm, sv, D->ownRows.p, nOwn,
+                   outC, bPartial_.p, bDots_.p, s, &launches_);
+    comm_.allReduceSum(bDots_.p, (size_t)bm, s);
+    borderRows(bDots_.p, bC0_.p, sv, bm, 0, bm, outC + nOwn, s, &launches_);
   };
-  auto Mglobal = [=](const double* inC, double* outFull) {
+  auto Mglobal = [=](const double* inC, double* outFull) {  // with a border: S -> bS_
     toGlobal(inC, gIn);
-    applyLevel0Dist(gIn, outFull);
+    applyLevel0Dist(gIn, outFull, bm ? inC + nOwn : nullptr);
     stats_.num_apply_inverse++;
   };
   auto A = [=](const double* inC, double* outC) {
     toGlobal(inC, gIn);
-    Aglobal(gIn, outC);
+    Aglobal(gIn, inC + nOwn, outC);
   };
   auto M = [=](const double* inC, double* outC) {
     Mglobal(inC, gOut);
     packIdx(gOut, D->ownRows.p, outC, nOwn, s, &launches_);
+    if (bm) HY_CUDA(cudaMemcpyAsync(outC + nOwn, bS_.p, bm * sizeof(double), cudaMemcpyDeviceToDevice, s));
   };
   L.A = A;
   L.M = M;
   L.dot = [=](const double* u, const double* v, double* d) {
-    multiDot(u, ld, 1, v, nOwn, kPartial_.p, d, 0, s, &launches_);
+    multiDot(u, ld, 1, v, dotRows, kPartial_.p, d, 0, s, &launches_);
     comm_.allReduceSum(d, 1, s);
   };
   L.step = [=](const double* v, double* w) {
     if (right) {  // the global result of M^-1 goes straight into the operator
       Mglobal(v, gOut);
-      Aglobal(gOut, w);
+      Aglobal(gOut, bS_.p, w);
     } else if (left) {
       A(v, kW_.p);
       M(kW_.p, w);
@@ -161,10 +176,12 @@ KrylovLayout Engine::ownerLayout(bool left, bool right) {
   L.load = [=](const double* src, double* dst, cudaMemcpyKind kind) {
     HY_CUDA(cudaMemcpyAsync(gOut, src, n * sizeof(double), kind, s));
     packIdx(gOut, D->ownRows.p, dst, nOwn, s, &launches_);
+    if (bm) HY_CUDA(cudaMemsetAsync(dst + nOwn, 0, bm * sizeof(double), s));
   };
-  L.keepOwn = [=](std::vector<double>& full) {
-    std::vector<double> own(nOwn);
+  L.keepOwn = [=](std::vector<double>& full) {  // n + m host numbers -> owned rows + border entries
+    std::vector<double> own(nOwn + bm);
     for (int64_t i = 0; i < nOwn; ++i) own[i] = full[D->hOwnRows[i]];
+    for (int j = 0; j < bm; ++j) own[nOwn + j] = full[n + j];
     full.swap(own);
   };
   L.store = [=](const double* src, double* dst, cudaMemcpyKind kind) {  // replicated, like the single-GPU entry point
@@ -286,7 +303,7 @@ void Engine::solve(const double* b, double* x, int where, uint64_t seed, hymls_b
       }
     }
   } else {
-    const int64_t ldV = L.rowLd, nloc = L.rows;
+    const int64_t ldV = L.rowLd, nloc = L.rows, nDot = L.dotRows;
     HY_CUDA(cudaMemsetAsync(kV_.p, 0, (size_t)(m + 1) * ldV * sizeof(double), s));
     std::vector<double> H((size_t)(m + 1) * m, 0.0), cs(m), sn(m), g(m + 1), hbuf(2 * m + 8);
     double* dH1 = kH_.p;              // first Gram-Schmidt pass  (m+1)
@@ -344,13 +361,13 @@ void Engine::solve(const double* b, double* x, int where, uint64_t seed, hymls_b
         L.step(vk, w);
         lap("operator step");
         // two passes of classical Gram-Schmidt (Belos ICGS/DGKS), fused multi-dot + multi-axpy
-        multiDot(kV_.p, ldV, k + 1, w, nloc, kPartial_.p, dH1, 0, s, &launches_);
+        multiDot(kV_.p, ldV, k + 1, w, nDot, kPartial_.p, dH1, 0, s, &launches_);
         comm_.allReduceSum(dH1, (size_t)(k + 1), s);
         multiAxpy(kV_.p, ldV, k + 1, dH1, w, nloc, -1.0, s, &launches_);
-        multiDot(kV_.p, ldV, k + 1, w, nloc, kPartial_.p, dH2, 0, s, &launches_);
+        multiDot(kV_.p, ldV, k + 1, w, nDot, kPartial_.p, dH2, 0, s, &launches_);
         comm_.allReduceSum(dH2, (size_t)(k + 1), s);
         multiAxpy(kV_.p, ldV, k + 1, dH2, w, nloc, -1.0, s, &launches_);
-        multiDot(w, ldV, 1, w, nloc, kPartial_.p, dNrm, 0, s, &launches_);
+        multiDot(w, ldV, 1, w, nDot, kPartial_.p, dNrm, 0, s, &launches_);
         comm_.allReduceSum(dNrm, 1, s);
         scaleByInvNorm(w, dNrm, w, nloc, s, &launches_);
         lap("CGS2 (4 sweeps, 3 allreduces)");

@@ -38,6 +38,9 @@ enum {
 /* where a vector/matrix argument lives */
 enum { HYMLS_B200_HOST = 0, HYMLS_B200_DEVICE = 1 };
 
+/* CUDA device the handle is bound to (the current device at hymls_b200_create); HYMLS_B200_ERR_CUDA without one. */
+int hymls_b200_get_device(hymls_b200_t* h);
+
 /* Message of the last failure on this thread ("" if none). */
 const char* hymls_b200_last_error(void);
 
@@ -124,6 +127,16 @@ int hymls_b200_apply_inverse(hymls_b200_t* h, const double* B, int64_t ldb, doub
 int64_t hymls_b200_owned_rows(hymls_b200_t* h, int64_t* rows, int64_t cap);
 int hymls_b200_local_rows(hymls_b200_t* h, int64_t* r0, int64_t* r1);
 int hymls_b200_apply_inverse_dist(hymls_b200_t* h, const double* B_local, double* X_local, int where);
+/*
+ * Bordered form on the same rows: [X; S] = [K V; W' C]^-1 [B; T] with B_local / X_local the rows of
+ * hymls_b200_owned_rows and T, S replicated m-vectors (S comes out bitwise equal on every rank); `where` applies to
+ * all four buffers.  Only separator values on the interfaces, the V-sums and a few m-vectors cross NVLink.  With one
+ * rank it is hymls_b200_apply_inverse_bordered.  hymls_b200_apply_inverse_dist with a border set means T = 0 with S
+ * discarded, as for hymls_b200_apply_inverse.  Without a border set m = 0: X is the plain ApplyInverse and S, which
+ * has no entries, is not written (as for hymls_b200_apply_inverse_bordered).
+ */
+int hymls_b200_apply_inverse_bordered_dist(hymls_b200_t* h, const double* B_local, const double* T, double* X_local,
+                                           double* S, int where);
 
 /*
  * Vectors in the CALLER's distribution (Epetra_Operator::ApplyInverse on the matrix' row map, any map):
@@ -150,6 +163,8 @@ int hymls_b200_set_border_dist(hymls_b200_t* h, int64_t n_local, const int64_t* 
  * Compute() must be called afterwards.
  */
 int hymls_b200_set_border(hymls_b200_t* h, const double* V, const double* W, const double* C, int m);
+/* m of the border set by hymls_b200_set_border / hymls_b200_set_border_dist (0: none) */
+int hymls_b200_border_size(hymls_b200_t* h);
 /* [X;S] = [K V; W' C]^-1 [B;T]  (Preconditioner.cpp:930-1070); T, S are m x nvec column major. */
 int hymls_b200_apply_inverse_bordered(hymls_b200_t* h, const double* B, int64_t ldb, const double* T,
                                       double* X, int64_t ldx, double* S, int nvec, int where);
@@ -163,7 +178,8 @@ int hymls_b200_apply_matrix(hymls_b200_t* h, const double* x, double* y, int whe
  * Preconditioning, Initial Vector Zero|Random|Previous, "Iterative Solver": Maximum Iterations,
  * Num Blocks, Maximum Restarts, Convergence Tolerance, Explicit Residual Test, *Residual Scaling).
  * x holds the initial guess when Initial Vector = Previous and receives the solution.
- * If a border is set the bordered system is solved (HYMLS::BorderedSolver) with right-hand side [b;0].
+ * If a border is set the bordered system is solved (HYMLS::BorderedSolver) with right-hand side [b;0], on several
+ * ranks on the owner distribution like the unbordered system (the m border entries are replicated on every rank).
  * resid_history (may be NULL) receives up to history_cap relative implicit residuals, iteration 0 first.
  */
 typedef struct {
@@ -233,6 +249,10 @@ typedef struct {
                                    than HYMLS_B200_HOST_PIPELINE_MIN_ROWS, default 2^20).  Used for pinned buffers only */
   int64_t host_pipeline_state;  /* 0: not used yet, 1: in use (its first call reproduced the serial path bit for bit),
                                    -1: that check failed, serial copies are used, -2: switched off (HYMLS_B200_HOST_PIPELINE=0) */
+  int64_t collective_calls;     /* NCCL calls of this rank since comm_init (all-reduce, broadcast, all-gather, one per grouped
+                                   neighbour exchange); 0 on one rank */
+  int64_t collective_bytes;     /* their payload on this rank: 8 * count of every all-reduce / broadcast / all-gather (one
+                                   rank's part), plus the bytes sent and received by the neighbour exchanges */
 } hymls_b200_stats;
 int hymls_b200_get_stats(hymls_b200_t* h, hymls_b200_stats* st);
 
