@@ -15,39 +15,66 @@ namespace hymls {
 
 // ---------------------------------------------------------------------------------------------
 // Batched dense mat-vec with the explicit inverses:  y_sd = Ainv_sd * x_sd  for every subdomain.
-// The dominant kernel of ApplyInverse: streams 8 n_sd^2 bytes per subdomain exactly once.
+// The dominant kernel of ApplyInverse: streams sizeof(T) n_sd^2 bytes per subdomain exactly once.
 // Work item = (matrix, slab of GEMV_ROWS rows); one warp per row, lanes stride the row with 16-byte
 // loads, x_sd staged in shared memory.
 //   x_sd[q] = xin[gather ? gather[p] : p] (- xsub[p]),  p = vecOff[mat] + q
 //   rows [0, nrows[mat]) only when nrows is given (the first solve of ApplyInverse needs a leading block)
 //   mode 0:  out[scatter ? scatter[p] : p] = acc
 //   mode 1:  out[scatter ? scatter[p] : p] = xprev[p] - acc   (second A11 solve of ApplyInverse: fused update + export)
+// T is the element type of the stored inverses: double, or float for a store narrowed by narrowToFloat ("Subdomain
+// Inverse Precision" = "Single", GemvArgs::A32).  A float entry is widened to double as it is loaded; x, the products
+// and the sums are FP64 in both.  A 16-byte load brings 2 doubles or 4 floats.
 // (Tried in round 2 and dropped: two rows per warp at a time -- 8 loads in flight per lane, x read once for both rows --
 //  needs 78 registers, 3 CTAs per SM instead of 4, and ran the full pass at 5.6 TB/s instead of 6.1 TB/s.)
 // ---------------------------------------------------------------------------------------------
 static constexpr int GEMV_ROWS = 32;   // rows per CTA
 static constexpr int GEMV_T = 256;     // 8 warps, 4 rows each
 
+template <typename T>
+__device__ __forceinline__ const T* gemvMatrix(const GemvArgs& a);
+template <>
+__device__ __forceinline__ const double* gemvMatrix<double>(const GemvArgs& a) { return a.A; }
+template <>
+__device__ __forceinline__ const float* gemvMatrix<float>(const GemvArgs& a) { return a.A32; }
+
+// Shared-memory slot of x_sd[q] in a segment of nc entries.  double: natural order, the pair (2k, 2k+1) beside the
+// double2 k of a row.  float: the float4 k of a row covers columns 4k..4k+3; their x values are kept as two arrays of
+// pairs, lo[k] = x[4k..4k+1] at 0 and hi[k] = x[4k+2..4k+3] at nc / 2, so that lane k reads two consecutive 16-byte
+// words (no bank conflicts, unlike the stride-32-byte reads of the natural order).  nc is a multiple of 4 for float.
+template <typename T>
+__device__ __forceinline__ int xSlot(int q, int nc) {
+  if constexpr (sizeof(T) == sizeof(double)) return q;
+  else return ((q >> 2) << 1) + (q & 1) + ((q & 2) ? (nc >> 1) : 0);
+}
+
+// one float4 of a row against its four x values (lo, hi as laid out by xSlot<float>), in double
+__device__ __forceinline__ double dot4(float4 m, double2 lo, double2 hi) {
+  return (double)m.x * lo.x + (double)m.y * lo.y + (double)m.z * hi.x + (double)m.w * hi.y;
+}
+
+template <typename T>
 __global__ void __launch_bounds__(GEMV_T)
 k_batched_gemv(GemvArgs a) {
+  constexpr int W = 16 / sizeof(T);  // entries per 16-byte load
   const int item = blockIdx.x;
   const int mat = a.itemMat[item];
   const int r0 = a.itemRow0[item];
   const int n = a.n[mat], np = a.np[mat];
   const int nr = a.nrows ? a.nrows[mat] : n;
   const int64_t v0 = a.vecOff[mat];  // offset of this matrix' segment in the packed vectors
-  const double* __restrict__ A = a.A + a.matOff[mat];
+  const T* __restrict__ A = gemvMatrix<T>(a) + a.matOff[mat];
   extern __shared__ double sx[];
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  // columns read: all (padded) np, or the leading ncols[mat] rounded up to a 16-byte pair
-  const int nc = a.ncols ? min(np, (a.ncols[mat] + 1) & ~1) : np;
+  // columns read: all (padded) np, or the leading ncols[mat] rounded up to one 16-byte load
+  const int nc = a.ncols ? min(np, (a.ncols[mat] + W - 1) & ~(W - 1)) : np;
   for (int q = tid; q < nc; q += GEMV_T) {
     double v = 0.0;
     if (q < n) {
       v = a.gather ? a.xin[a.gather[v0 + q]] : a.xin[v0 + q];
       if (a.xsub) v -= a.xsub[v0 + q];
     }
-    sx[q] = v;
+    sx[xSlot<T>(q, nc)] = v;
   }
   __syncthreads();
   // rows per warp: 4 (a 32-row slab per CTA) unless the work list was built with thinner slabs (a.rowsPerWarp:
@@ -56,22 +83,36 @@ k_batched_gemv(GemvArgs a) {
   for (int rr = 0; rr < rpw; ++rr) {
     const int r = r0 + wid * rpw + rr;
     if (r >= nr) break;
-    const double2* __restrict__ row = reinterpret_cast<const double2*>(A + (int64_t)r * np);
-    const double2* __restrict__ x2 = reinterpret_cast<const double2*>(sx);
     double acc0 = 0.0, acc1 = 0.0;
-    const int n2 = nc >> 1;
-    int q = lane;
-    for (; q + 96 < n2; q += 128) {  // 4 independent 16-byte loads in flight per lane
-      double2 m0 = __ldg(row + q), m1 = __ldg(row + q + 32), m2 = __ldg(row + q + 64), m3 = __ldg(row + q + 96);
-      double2 b0 = x2[q], b1 = x2[q + 32], b2 = x2[q + 64], b3 = x2[q + 96];
-      acc0 += m0.x * b0.x + m1.x * b1.x + m2.x * b2.x + m3.x * b3.x;
-      acc1 += m0.y * b0.y + m1.y * b1.y + m2.y * b2.y + m3.y * b3.y;
-    }
-    for (; q < n2; q += 32) {
-      double2 m0 = __ldg(row + q);
-      double2 b0 = x2[q];
-      acc0 += m0.x * b0.x;
-      acc1 += m0.y * b0.y;
+    if constexpr (W == 2) {
+      const double2* __restrict__ row = reinterpret_cast<const double2*>(A + (int64_t)r * np);
+      const double2* __restrict__ x2 = reinterpret_cast<const double2*>(sx);
+      const int n2 = nc >> 1;
+      int q = lane;
+      for (; q + 96 < n2; q += 128) {  // 4 independent 16-byte loads in flight per lane
+        double2 m0 = __ldg(row + q), m1 = __ldg(row + q + 32), m2 = __ldg(row + q + 64), m3 = __ldg(row + q + 96);
+        double2 b0 = x2[q], b1 = x2[q + 32], b2 = x2[q + 64], b3 = x2[q + 96];
+        acc0 += m0.x * b0.x + m1.x * b1.x + m2.x * b2.x + m3.x * b3.x;
+        acc1 += m0.y * b0.y + m1.y * b1.y + m2.y * b2.y + m3.y * b3.y;
+      }
+      for (; q < n2; q += 32) {
+        double2 m0 = __ldg(row + q);
+        double2 b0 = x2[q];
+        acc0 += m0.x * b0.x;
+        acc1 += m0.y * b0.y;
+      }
+    } else {
+      const float4* __restrict__ row = reinterpret_cast<const float4*>(A + (int64_t)r * np);
+      const double2* __restrict__ lo = reinterpret_cast<const double2*>(sx);
+      const double2* __restrict__ hi = reinterpret_cast<const double2*>(sx + (nc >> 1));
+      const int n4 = nc >> 2;
+      int q = lane;
+      for (; q + 96 < n4; q += 128) {  // 4 independent 16-byte loads in flight per lane
+        float4 m0 = __ldg(row + q), m1 = __ldg(row + q + 32), m2 = __ldg(row + q + 64), m3 = __ldg(row + q + 96);
+        acc0 += dot4(m0, lo[q], hi[q]) + dot4(m1, lo[q + 32], hi[q + 32]);
+        acc1 += dot4(m2, lo[q + 64], hi[q + 64]) + dot4(m3, lo[q + 96], hi[q + 96]);
+      }
+      for (; q < n4; q += 32) acc0 += dot4(__ldg(row + q), lo[q], hi[q]);
     }
     double acc = acc0 + acc1;
 #pragma unroll
@@ -84,14 +125,20 @@ k_batched_gemv(GemvArgs a) {
   }
 }
 
+template <typename T>
+static void launchGemv(const GemvArgs& a, int numItems, size_t smem, cudaStream_t s) {
+  static PerDeviceLimit limit;
+  if (limit.raise(smem))
+    HY_CUDA(cudaFuncSetAttribute(k_batched_gemv<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_batched_gemv<T><<<numItems, GEMV_T, smem, s>>>(a);
+}
+
 void batchedGemv(const GemvArgs& a, int numItems, int npMax, cudaStream_t s, int64_t* launches) {
   if (numItems == 0) return;
-  static PerDeviceLimit limit;
   size_t smem = (size_t)npMax * sizeof(double);
   if (smem > 227 * 1024) throw Error(HYMLS_B200_ERR_UNSUPPORTED, "dense block too large for the GEMV kernel");
-  if (limit.raise(smem))
-    HY_CUDA(cudaFuncSetAttribute(k_batched_gemv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_batched_gemv<<<numItems, GEMV_T, smem, s>>>(a);
+  if (a.A32) launchGemv<float>(a, numItems, smem, s);
+  else launchGemv<double>(a, numItems, smem, s);
   ++*launches;
 }
 int gemvRowsPerItem() { return GEMV_ROWS; }
@@ -235,7 +282,7 @@ bool smallGemv(const GemvArgs& a, const int* matList, int numMats, int npMax, cu
 // ONCE and multiplied with NV vectors staged in shared memory, so k columns cost one pass over the inverses instead
 // of k.  Vector v of xin / xsub / out starts at v * ldIn / ldSub / ldOut.  mode 0 only.
 // ---------------------------------------------------------------------------------------------
-template <int NV>
+template <typename T, int NV>
 __global__ void __launch_bounds__(GEMV_T)
 k_batched_gemv_multi(GemvArgs a, int64_t ldIn, int64_t ldSub, int64_t ldOut) {
   const int item = blockIdx.x;
@@ -244,7 +291,7 @@ k_batched_gemv_multi(GemvArgs a, int64_t ldIn, int64_t ldSub, int64_t ldOut) {
   const int n = a.n[mat], np = a.np[mat];
   const int nr = a.nrows ? a.nrows[mat] : n;
   const int64_t v0 = a.vecOff[mat];
-  const double* __restrict__ A = a.A + a.matOff[mat];
+  const T* __restrict__ A = gemvMatrix<T>(a) + a.matOff[mat];
   extern __shared__ double sx[];  // NV x np
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   for (int q = tid; q < np; q += GEMV_T) {
@@ -256,7 +303,7 @@ k_batched_gemv_multi(GemvArgs a, int64_t ldIn, int64_t ldSub, int64_t ldOut) {
         x = a.xin[v * ldIn + src];
         if (a.xsub) x -= a.xsub[v * ldSub + v0 + q];
       }
-      sx[v * np + q] = x;
+      sx[v * np + xSlot<T>(q, np)] = x;
     }
   }
   __syncthreads();
@@ -264,27 +311,51 @@ k_batched_gemv_multi(GemvArgs a, int64_t ldIn, int64_t ldSub, int64_t ldOut) {
   for (int rr = 0; rr < GEMV_ROWS / (GEMV_T / 32); ++rr) {
     const int r = r0 + wid * (GEMV_ROWS / (GEMV_T / 32)) + rr;
     if (r >= nr) break;
-    const double2* __restrict__ row = reinterpret_cast<const double2*>(A + (int64_t)r * np);
     double acc[NV];
 #pragma unroll
     for (int v = 0; v < NV; ++v) acc[v] = 0.0;
-    const int n2 = np >> 1;
-    int q = lane;
-    for (; q + 32 < n2; q += 64) {  // two independent 16-byte loads in flight per lane
-      const double2 m0 = __ldg(row + q), m1 = __ldg(row + q + 32);
+    if constexpr (sizeof(T) == sizeof(double)) {
+      const double2* __restrict__ row = reinterpret_cast<const double2*>(A + (int64_t)r * np);
+      const int n2 = np >> 1;
+      int q = lane;
+      for (; q + 32 < n2; q += 64) {  // two independent 16-byte loads in flight per lane
+        const double2 m0 = __ldg(row + q), m1 = __ldg(row + q + 32);
 #pragma unroll
-      for (int v = 0; v < NV; ++v) {
-        const double2 b0 = reinterpret_cast<const double2*>(sx + v * np)[q];
-        const double2 b1 = reinterpret_cast<const double2*>(sx + v * np)[q + 32];
-        acc[v] += m0.x * b0.x + m0.y * b0.y + m1.x * b1.x + m1.y * b1.y;
+        for (int v = 0; v < NV; ++v) {
+          const double2 b0 = reinterpret_cast<const double2*>(sx + v * np)[q];
+          const double2 b1 = reinterpret_cast<const double2*>(sx + v * np)[q + 32];
+          acc[v] += m0.x * b0.x + m0.y * b0.y + m1.x * b1.x + m1.y * b1.y;
+        }
       }
-    }
-    for (; q < n2; q += 32) {
-      const double2 m0 = __ldg(row + q);
+      for (; q < n2; q += 32) {
+        const double2 m0 = __ldg(row + q);
 #pragma unroll
-      for (int v = 0; v < NV; ++v) {
-        const double2 b0 = reinterpret_cast<const double2*>(sx + v * np)[q];
-        acc[v] += m0.x * b0.x + m0.y * b0.y;
+        for (int v = 0; v < NV; ++v) {
+          const double2 b0 = reinterpret_cast<const double2*>(sx + v * np)[q];
+          acc[v] += m0.x * b0.x + m0.y * b0.y;
+        }
+      }
+    } else {
+      const float4* __restrict__ row = reinterpret_cast<const float4*>(A + (int64_t)r * np);
+      const int n4 = np >> 2;
+      int q = lane;
+      for (; q + 32 < n4; q += 64) {  // two independent 16-byte loads in flight per lane
+        const float4 m0 = __ldg(row + q), m1 = __ldg(row + q + 32);
+#pragma unroll
+        for (int v = 0; v < NV; ++v) {
+          const double2* lo = reinterpret_cast<const double2*>(sx + v * np);
+          const double2* hi = reinterpret_cast<const double2*>(sx + v * np + (np >> 1));
+          acc[v] += dot4(m0, lo[q], hi[q]) + dot4(m1, lo[q + 32], hi[q + 32]);
+        }
+      }
+      for (; q < n4; q += 32) {
+        const float4 m0 = __ldg(row + q);
+#pragma unroll
+        for (int v = 0; v < NV; ++v) {
+          const double2* lo = reinterpret_cast<const double2*>(sx + v * np);
+          const double2* hi = reinterpret_cast<const double2*>(sx + v * np + (np >> 1));
+          acc[v] += dot4(m0, lo[q], hi[q]);
+        }
       }
     }
 #pragma unroll
@@ -303,25 +374,50 @@ k_batched_gemv_multi(GemvArgs a, int64_t ldIn, int64_t ldSub, int64_t ldOut) {
   }
 }
 
+template <typename T, int NV>
+static void launchGemvMulti(const GemvArgs& a, int numItems, size_t smem, int64_t ldIn, int64_t ldSub, int64_t ldOut,
+                            cudaStream_t s) {
+  static PerDeviceLimit limit;
+  if (limit.raise(smem))
+    HY_CUDA(cudaFuncSetAttribute(k_batched_gemv_multi<T, NV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_batched_gemv_multi<T, NV><<<numItems, GEMV_T, smem, s>>>(a, ldIn, ldSub, ldOut);
+}
+template <typename T>
+static void launchGemvMulti(const GemvArgs& a, int numItems, size_t smem, int nv, int64_t ldIn, int64_t ldSub,
+                            int64_t ldOut, cudaStream_t s) {
+  if (nv == 2) launchGemvMulti<T, 2>(a, numItems, smem, ldIn, ldSub, ldOut, s);
+  else if (nv == 3) launchGemvMulti<T, 3>(a, numItems, smem, ldIn, ldSub, ldOut, s);
+  else launchGemvMulti<T, 4>(a, numItems, smem, ldIn, ldSub, ldOut, s);
+}
+
 // nv in 2..4; returns false when the kernel cannot hold nv vectors of npMax entries in shared memory
 bool batchedGemvMulti(const GemvArgs& a, int numItems, int npMax, int nv, int64_t ldIn, int64_t ldSub, int64_t ldOut,
                       cudaStream_t s, int64_t* launches) {
   if (numItems == 0) return true;
   const size_t smem = (size_t)npMax * nv * sizeof(double);
   if (smem > 200 * 1024 || nv < 2 || nv > 4) return false;
-  static PerDeviceLimit lim2, lim3, lim4;
-  if (nv == 2) {
-    if (lim2.raise(smem)) HY_CUDA(cudaFuncSetAttribute(k_batched_gemv_multi<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_batched_gemv_multi<2><<<numItems, GEMV_T, smem, s>>>(a, ldIn, ldSub, ldOut);
-  } else if (nv == 3) {
-    if (lim3.raise(smem)) HY_CUDA(cudaFuncSetAttribute(k_batched_gemv_multi<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_batched_gemv_multi<3><<<numItems, GEMV_T, smem, s>>>(a, ldIn, ldSub, ldOut);
-  } else {
-    if (lim4.raise(smem)) HY_CUDA(cudaFuncSetAttribute(k_batched_gemv_multi<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_batched_gemv_multi<4><<<numItems, GEMV_T, smem, s>>>(a, ldIn, ldSub, ldOut);
-  }
+  if (a.A32) launchGemvMulti<float>(a, numItems, smem, nv, ldIn, ldSub, ldOut, s);
+  else launchGemvMulti<double>(a, numItems, smem, nv, ldIn, ldSub, ldOut, s);
   ++*launches;
   return true;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Narrowing of a "Single" store: dst[i] = (float)src[i], round to nearest even.  A finite entry that becomes
+// infinite (|x| above FLT_MAX after rounding) sets *overflow = 1; entries that are already Inf / NaN stay so silently.
+// ---------------------------------------------------------------------------------------------
+__global__ void k_narrow_to_float(const double* __restrict__ src, float* __restrict__ dst, int64_t n, int* overflow) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const double v = src[i];
+    const float f = __double2float_rn(v);
+    if (isinf(f) && isfinite(v)) *overflow = 1;
+    dst[i] = f;
+  }
+}
+void narrowToFloat(const double* src, float* dst, int64_t n, int* overflow, cudaStream_t s, int64_t* launches) {
+  if (n == 0) return;
+  k_narrow_to_float<<<(unsigned)std::min<int64_t>((n + 255) / 256, 148 * 16), 256, 0, s>>>(src, dst, n, overflow);
+  ++*launches;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -784,6 +880,7 @@ k_batched_gemv_t(GemvArgs a, int tilesPerMat) {
   if (j < n) a.out[v0 + j] = acc;
 }
 void batchedGemvT(const GemvArgs& a, int count, int npMax, cudaStream_t s, int64_t* launches) {
+  if (a.A32) throw Error(HYMLS_B200_ERR_STATE, "batchedGemvT: the inverses have been narrowed to FP32");
   if (count == 0 || npMax == 0) return;
   const int tiles = (npMax + 255) / 256;
   k_batched_gemv_t<<<(unsigned)(count * tiles), 256, 0, s>>>(a, tiles);

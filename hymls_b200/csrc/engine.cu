@@ -30,7 +30,7 @@ static void validatePreconditionerList(const ParameterList& prec) {
       "Separator Length (y)", "Separator Length (z)", "Subdivide Separators", "Subdivide based on variable",
       "Subdomain Solver Num Threads", "Subdomain Solver Type", "Visualize Solver",
       // extension of this implementation (DESIGN.md, "Deviations")
-      "Eliminate Tube Pressures With Velocities", "Refine Inverses"};
+      "Eliminate Tube Pressures With Velocities", "Refine Inverses", "Subdomain Inverse Precision"};
   for (const std::string& name : prec.parameterNames()) {
     bool ok = startsWith(name, "Fix GID ") || startsWith(name, "Retain Nodes");
     for (const char* v : valid) ok = ok || name == v;
@@ -74,6 +74,15 @@ void Engine::readParameters() {
   // extension: one Newton-Schulz step on every explicit inverse (DESIGN.md, parity section); default on
   refine_ = prec.get("Refine Inverses", true);
   if (const char* e = getenv("HYMLS_B200_REFINE")) refine_ = atoi(e) != 0;
+  // extension: FP32 storage of the subdomain inverses (DESIGN.md, Deviations); the default is not written back, so the
+  // final list of a run that does not name the parameter stays as it was
+  singleInverses_ = false;
+  if (prec.isParameter("Subdomain Inverse Precision")) {
+    const std::string p = prec.get("Subdomain Inverse Precision", "Double");  // a value that is no string throws
+    if (p != "Double" && p != "Single")
+      throw Error(HYMLS_B200_ERR_ARG, "Subdomain Inverse Precision '" + p + "': valid values are 'Double' and 'Single'");
+    singleInverses_ = p == "Single";
+  }
   std::string method = prec.get("Partitioner", "Cartesian");
   if (method != "Cartesian" && method != "Skew Cartesian")
     throw Error(HYMLS_B200_ERR_ARG, "Partitioner '" + method + "': Up to now we only support Cartesian partitioning");
@@ -280,6 +289,7 @@ void BatchedInverse::setup(const std::vector<int>& n_, const std::vector<int>& n
   itemMat.upload(im, s);
   itemRow0.upload(ir, s);
   F.alloc((size_t)(count ? matOff_[count] : 0));
+  narrowed = false;
   HY_CUDA(cudaStreamSynchronize(s));
 }
 GemvArgs BatchedInverse::args() const {
@@ -290,7 +300,8 @@ GemvArgs BatchedInverse::args() const {
   a.np = np.p;
   a.matOff = matOff.p;
   a.vecOff = vecOff.p;
-  a.A = F.p;
+  if (narrowed) a.A32 = reinterpret_cast<const float*>(F.p);
+  else a.A = F.p;
   a.rowsPerWarp = rowsPerWarp;
   return a;
 }
@@ -794,14 +805,15 @@ void Engine::uploadLevel(Level& L) {
 // ---------------------------------------------------------------------------------------------
 // Compute
 // ---------------------------------------------------------------------------------------------
-// Collective when sharded: every rank learns whether ANY rank met a zero pivot, so that all of them leave
-// Compute with the same error instead of one rank throwing while the others wait in the next collective.
-void Engine::checkInfo(const std::string& what) {
+// Collective when sharded: every rank learns whether ANY rank set info_ (a zero pivot, a narrowing overflow), so that
+// all of them leave Compute with the same error instead of one rank throwing while the others wait in the next
+// collective.  Returns this rank's info_; *elsewhere: set on another rank only.
+int Engine::infoOnAnyRank(bool* elsewhere) {
   cudaStream_t s = stream_;
   int h = 0;
   HY_CUDA(cudaMemcpyAsync(&h, info_.p, sizeof(int), cudaMemcpyDeviceToHost, s));
   HY_CUDA(cudaStreamSynchronize(s));
-  bool elsewhere = false;
+  *elsewhere = false;
   if (comm_.active()) {
     flag_.alloc(1);
     double f = h != 0 ? 1.0 : 0.0;
@@ -809,13 +821,46 @@ void Engine::checkInfo(const std::string& what) {
     comm_.allReduceSum(flag_.p, 1, s);
     HY_CUDA(cudaMemcpyAsync(&f, flag_.p, sizeof(double), cudaMemcpyDeviceToHost, s));
     HY_CUDA(cudaStreamSynchronize(s));
-    elsewhere = (f != 0.0 && h == 0);
+    *elsewhere = (f != 0.0 && h == 0);
   }
+  return h;
+}
+
+void Engine::checkInfo(const std::string& what) {
+  bool elsewhere = false;
+  const int h = infoOnAnyRank(&elsewhere);
   if (h != 0 || elsewhere)
     throw Error(HYMLS_B200_ERR_NUMERIC,
                 what + ": zero pivot (" + (elsewhere ? std::string("on another rank") : "matrix " + std::to_string(h - 1)) +
                     " is exactly singular). For 3D Stokes-C on the Cartesian partitioner the reference's pressure "
                     "'tube' blocks are identically zero; see 'Eliminate Tube Pressures With Velocities' in DESIGN.md");
+}
+
+// "Subdomain Inverse Precision" = "Single": rounds the FP64 inverses of level l to FP32 (nearest even) in place, after
+// the last reader of the FP64 store in Compute.  The float of entry i goes to float index i, so matOff / vecOff and the
+// GEMV work lists stay as they are; ApplyInverse reads them through GemvArgs::A32.  The next Compute writes FP64 again.
+void Engine::narrowA11(int l) {
+  Level& L = *levels_[l];
+  cudaStream_t s = stream_;
+  HY_CUDA(cudaMemsetAsync(info_.p, 0, sizeof(int), s));
+  float* dst = reinterpret_cast<float*>(L.a11.F.p);
+  // Chunk by chunk through work_ (it holds at least one a11Chunks chunk): all of chunk [o0, o1) is converted into
+  // work_ first, then copied to bytes [4 o0, 4 o1) of the store.  Those bytes lie in doubles [o0 / 2, o1 / 2), i.e.
+  // in this chunk or earlier ones, which have been read already: the order is safe for any chunk size.
+  for (const auto& ch : a11Chunks(L)) {
+    const int64_t o0 = L.ownOff[ch.first], o1 = L.ownOff[ch.second];
+    work_.alloc((size_t)(o1 - o0));
+    float* w = reinterpret_cast<float*>(work_.p);
+    narrowToFloat(L.a11.F.p + o0, w, o1 - o0, info_.p, s, &launches_);
+    HY_CUDA(cudaMemcpyAsync(dst + o0, w, (size_t)(o1 - o0) * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  }
+  L.a11.narrowed = true;
+  bool elsewhere = false;
+  if (infoOnAnyRank(&elsewhere) != 0 || elsewhere)
+    throw Error(HYMLS_B200_ERR_NUMERIC,
+                "subdomain solver (A11) of level " + std::to_string(l) + ": an entry of the inverse exceeds the FP32 " +
+                    "range" + (elsewhere ? " on another rank" : "") +
+                    "; use 'Subdomain Inverse Precision' = 'Double' for this matrix");
 }
 
 void Engine::needComm() const {
@@ -834,7 +879,10 @@ void Engine::compute() {
   info_.alloc(1);
   HY_CUDA(cudaMemsetAsync(info_.p, 0, sizeof(int), stream_));
   stats_.flops_compute = 0;
-  for (int l = 0; l < (int)levels_.size(); ++l) computeLevel(l);
+  for (int l = 0; l < (int)levels_.size(); ++l) {
+    computeLevel(l);
+    if (singleInverses_) narrowA11(l);  // computeLevel(l) is the last reader of the FP64 store of level l
+  }
   HY_CUDA(cudaEventRecord(ev1_, stream_));
   HY_CUDA(cudaStreamSynchronize(stream_));
   float ms = 0;
@@ -1056,6 +1104,7 @@ void Engine::computeLevel(int l) {
   LevelSym& S = L.sym;
   cudaStream_t s = stream_;
   PhaseTimer pt(s, l);
+  L.a11.narrowed = false;  // the inversion below writes FP64 values over a narrowed store of the previous Compute
   // (1) off-diagonal blocks: value gathers (MatrixBlock::Compute)
   gatherValues(L.val.p, L.src12.p, L.v12.p, L.nnz12, s, &launches_);
   gatherValues(L.val.p, L.src21.p, L.v21.p, (int64_t)L.v21.n, s, &launches_);
@@ -2196,6 +2245,16 @@ int64_t Engine::debugCopy(int level, const std::string& name, double* out, int64
   Level& L = *levels_.at(level);
   const double* p = nullptr;
   int64_t n = 0;
+  if (name == "a11inv" && L.a11.narrowed) {  // the FP32 values, widened to double (same length)
+    n = (int64_t)L.a11.F.n;
+    if (out && cap >= n && n > 0) {
+      std::vector<float> f(n);
+      HY_CUDA(cudaMemcpyAsync(f.data(), L.a11.F.p, n * sizeof(float), cudaMemcpyDeviceToHost, stream_));
+      HY_CUDA(cudaStreamSynchronize(stream_));
+      std::copy(f.begin(), f.end(), out);
+    }
+    return n;
+  }
   if (name == "a11inv") { p = L.a11.F.p; n = (int64_t)L.a11.F.n; }
   else if (name == "blkinv") { p = L.blk.F.p; n = (int64_t)L.blk.F.n; }
   else if (name == "coarseinv") { p = coarse_.F.p; n = (int64_t)coarse_.F.n; }
@@ -2231,6 +2290,8 @@ int64_t Engine::debugCopy(int level, const std::string& name, double* out, int64
 void Engine::getStats(hymls_b200_stats* st) {
   *st = stats_;
   st->kernel_launches = launches_;
+  const double eb = singleInverses_ ? 4.0 : 8.0;  // bytes per stored A11^-1 entry
+  st->a11_entry_bytes = (int64_t)eb;
   if (!levels_.empty() && initialized_) {
     const LevelSym& S = levels_[0]->sym;
     st->n = S.n;
@@ -2252,17 +2313,17 @@ void Engine::getStats(hymls_b200_stats* st) {
       st->a11_split = splitActive(*levels_[0], 0) ? 1 : 0;
       st->host_pipeline_chunks = pipePlan_.K;
       st->host_pipeline_state = pipeEnabled_ ? pipeState_ : -2;
-      st->bytes_a11_full_pass = 8.0 * (st->a11_split ? ownLead : own);  // this rank's share when sharded
-      st->bytes_a11_level0 = 8.0 * (own + ownLead);
+      st->bytes_a11_full_pass = eb * (st->a11_split ? ownLead : own);  // this rank's share when sharded
+      st->bytes_a11_level0 = eb * (own + ownLead);
     }
     // SURVEY 8(d): algorithmic bytes of one ApplyInverse, summed over the levels; the A11 term is
-    // 8 (sum n^2 + sum n nb) since the first solve needs only the leading nb rows of every inverse
+    // eb (sum n^2 + sum n nb) since the first solve needs only the leading nb rows of every inverse
     double bytes = 0;
     for (auto& lp : levels_) {
       const LevelSym& T = lp->sym;
       double sb = 0;
       for (int b = 0; b < T.nblk; ++b) sb += 8.0 * (double)T.blkN[b] * T.blkN[b];
-      bytes += 8.0 * (T.sumNsq + T.sumNNb) + 12.0 * (double)(lp->nnz12 + lp->nnz21) +
+      bytes += eb * (T.sumNsq + T.sumNNb) + 12.0 * (double)(lp->nnz12 + lp->nnz21) +
                4.0 * (double)(T.nI + T.nS + 2) + sb + 2.0 * 12.0 * (double)T.nS * 2.0 + 8.0 * (10.0 * T.nI + 14.0 * T.nS);
     }
     if (coarseBT_.active) {

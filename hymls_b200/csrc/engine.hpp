@@ -13,6 +13,7 @@ namespace hymls {
 
 struct BatchedInverse {  // a set of dense inverses + the GEMV work list over them
   DevBuf<double> F;
+  bool narrowed = false;  // F holds FP32 values (float index = double index, Engine::narrowA11); set by Compute
   DevBuf<int> n, np, itemMat, itemRow0;
   DevBuf<int64_t> matOff, vecOff;
   std::vector<int> hN, hNp;
@@ -220,6 +221,8 @@ class Engine {
   void reserveComputeScratch();
   size_t inversionWorkspace() const;
   void checkInfo(const std::string& what);
+  int infoOnAnyRank(bool* elsewhere);
+  void narrowA11(int l);
   void computeCoarse(const int64_t* ptr, const int* col, double* val, int n, const std::vector<gidx>& rowGid,
                      const std::vector<int64_t>& hPtr, const std::vector<int>& hCol, const double* bV = nullptr,
                      const double* bW = nullptr, const std::vector<double>* bC = nullptr);
@@ -280,6 +283,7 @@ class Engine {
   DevBuf<double> work_;      // inversion workspace
   DevBuf<double> work2_, blkA_, blkR_;  // Newton-Schulz refinement: residuals, copies of the dense originals
   bool refine_ = true;
+  bool singleInverses_ = false;  // "Subdomain Inverse Precision" = "Single": A11 inverses stored in FP32 after Compute
   DevBuf<int> piv_, perm_, info_, subsetN_, subsetNp_;
   DevBuf<double> wsC_, wsSV_, wsSLL_, diagScratch_, blkW_, red2_, blk2_, a21d_, dmat_, a12d_, skd_;
   DevBuf<int64_t> relOff_;

@@ -106,6 +106,7 @@ struct GemvArgs {
   const int* nrows;        // optional: only rows [0, nrows[mat]) are computed (default: all n)
   const int* ncols;        // optional: x is zero beyond its first ncols[mat] entries, the rows are read that far only
   const double* A;
+  const float* A32;        // optional: the matrices stored in FP32 (narrowToFloat); when set, A is not read
   const double* xin;
   const int* gather;
   const double* xsub;      // optional: x_sd[q] = xin[...] - xsub[p]
@@ -125,6 +126,8 @@ bool batchedGemvMulti(const GemvArgs& a, int numItems, int npMax, int nv, int64_
 void ctaGemv(const GemvArgs& a, const int* matList, int numMats, int npMax, cudaStream_t s, int64_t* launches);
 bool smallGemv(const GemvArgs& a, const int* matList, int numMats, int npMax, cudaStream_t s, int64_t* launches);
 int gemvRowsPerItem();
+// dst[i] = (float)src[i] (round to nearest even) for i in [0, n); *overflow = 1 where a finite entry becomes infinite
+void narrowToFloat(const double* src, float* dst, int64_t n, int* overflow, cudaStream_t s, int64_t* launches);
 void spmv(const int64_t* ptr, const int* col, const double* val, const double* x, double* y, int64_t n, double alpha,
           const double* b, const int* bidx, double beta, cudaStream_t s, int64_t* launches);
 // indexing.cu: index arrays built on the device from the pattern
@@ -200,7 +203,8 @@ void gatherAddList(const double* b, const int* bidx, const double* t, double* y,
 void putDirichletCsr(double* val, const int64_t* ptr, const int* col, int row, cudaStream_t s, int64_t* launches);
 
 // ---- bordered variant (apply.cu) ----
-void batchedGemvT(const GemvArgs& a, int count, int npMax, cudaStream_t s, int64_t* launches);  // out = Ainv^T x
+// out = Ainv^T x on an FP64 store (Compute only; refuses A32)
+void batchedGemvT(const GemvArgs& a, int count, int npMax, cudaStream_t s, int64_t* launches);
 // y = alpha A^T x through a host-built transposed index into A's values (deterministic: no atomics)
 void spmvIndexed(const int64_t* ptr, const int* col, const int64_t* idx, const double* val, const double* x, double* y,
                  int64_t n, double alpha, cudaStream_t s, int64_t* launches);

@@ -228,12 +228,13 @@ typedef struct {
   double bytes_apply;           /* algorithmic bytes of one ApplyInverse (all levels), SURVEY 8(d) formula */
   double flops_compute;         /* algorithmic flops of Compute (inversions: 2 n^3) */
   double bytes_a11_level0;      /* this rank's level-0 A11^-1 bytes streamed by one ApplyInverse:
-                                   8 * sum (n_sd^2 + n_sd * nb_sd), full second solve + leading rows of the first */
+                                   a11_entry_bytes * sum (n_sd^2 + n_sd * nb_sd), full second solve + leading rows of
+                                   the first */
   int64_t kernel_launches;      /* launches issued by this handle so far */
   double device_bytes;          /* device memory held */
   double sum_nsd_nb;            /* sum n_sd * nb_sd (level 0): nb_sd = interior nodes that separator rows couple to;
                                    the first subdomain solve of ApplyInverse needs only these rows of A11^-1 */
-  double bytes_a11_full_pass;   /* this rank's 8 * sum n_sd^2: one full pass over its level-0 inverses */
+  double bytes_a11_full_pass;   /* this rank's a11_entry_bytes * sum n_sd^2: one full pass over its level-0 inverses */
   double ms_a11_lead;           /* set by hymls_b200_time_apply: CUDA-event time of the leading-rows pass */
   int64_t interior_couplings;   /* matrix entries between interiors of DIFFERENT subdomains, all levels: must be 0
                                    for a correct domain decomposition (Tester::isDDcorrect, src/HYMLS_Tester.cpp:253-455);
@@ -242,7 +243,8 @@ typedef struct {
                                    run on a low-priority stream beside the separator phase, and the pass on the critical
                                    path reads only the leading nb COLUMNS (x1 = A11^-1 b1 - A11^-1[:, :nb] (A12 x2)); the
                                    bytes per ApplyInverse are unchanged.  bytes_a11_full_pass / ms_a11_kernel_per_launch
-                                   then describe that leading-columns pass (8 * sum n_sd nb_sd bytes).  0: one full pass */
+                                   then describe that leading-columns pass (a11_entry_bytes * sum n_sd nb_sd bytes).
+                                   0: one full pass */
   int64_t host_pipeline_chunks; /* ApplyInverse with HOST buffers on one GPU: number of chunks in which the copy of b is
                                    overlapped with the leading-rows pass and the copy of x with the full pass over the
                                    level-0 inverses (0: no schedule -- several ranks, Number of Levels = 0, or fewer rows
@@ -253,6 +255,9 @@ typedef struct {
                                    neighbour exchange); 0 on one rank */
   int64_t collective_bytes;     /* their payload on this rank: 8 * count of every all-reduce / broadcast / all-gather (one
                                    rank's part), plus the bytes sent and received by the neighbour exchanges */
+  int64_t a11_entry_bytes;      /* bytes per stored entry of the subdomain inverses A11^-1 that ApplyInverse streams: 8, or 4
+                                   with "Subdomain Inverse Precision" = "Single" (FP32 storage, FP64 arithmetic).
+                                   bytes_a11_level0, bytes_a11_full_pass and the A11 term of bytes_apply count this many */
 } hymls_b200_stats;
 int hymls_b200_get_stats(hymls_b200_t* h, hymls_b200_stats* st);
 
