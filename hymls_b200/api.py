@@ -90,6 +90,8 @@ def load_library():
     lib.hymls_b200_apply_inverse_bordered.argtypes = [vp, vp, i64, vp, vp, i64, vp, C.c_int, C.c_int]
     lib.hymls_b200_apply_matrix.argtypes = [vp, vp, vp, C.c_int]
     lib.hymls_b200_solve.argtypes = [vp, vp, vp, C.c_int, C.c_uint64, P(_SolveInfo), vp, C.c_int]
+    lib.hymls_b200_solve_dist.argtypes = [vp, vp, vp, vp, vp, C.c_int, C.c_uint64, P(_SolveInfo), vp, C.c_int]
+    lib.hymls_b200_solve_map.argtypes = [vp, vp, vp, vp, vp, C.c_int, C.c_uint64, P(_SolveInfo), vp, C.c_int]
     lib.hymls_b200_set_tolerance.argtypes = [vp, C.c_double]
     lib.hymls_b200_get_parameters_xml.argtypes = [vp, C.c_char_p, i64]
     lib.hymls_b200_get_parameters_xml.restype = i64
@@ -495,10 +497,73 @@ class Solver:
             xc = torch.zeros_like(b) if x is None else x
             _check(lib, lib.hymls_b200_solve(P._h, b.data_ptr(), xc.data_ptr(), DEVICE, seed, C.byref(info),
                                              hist.ctypes.data, history_cap))
+        self._keep_info(info, hist, history_cap)
+        return xc
+
+    def _keep_info(self, info, hist, history_cap):
         self.num_iter = info.iterations
         self.info = {k: getattr(info, k) for k, _ in _SolveInfo._fields_}
         self.history = hist[:min(info.history_len, history_cap)].copy()
-        return xc
+
+    def ApplyInverseDist(self, b_local, T=None, x=None, seed=43, history_cap=2048):
+        """The Krylov solve on the rows of OwnedRows(), in that order: b_local in, x_local out (x, when given, holds
+        the initial guess for Initial Vector = Previous and receives the solution).  With a border set (m > 0) the
+        bordered system [K V; W' C] [x; s] = [b; T] is solved (T = None: T = 0) and (x_local, S) is returned, S bitwise
+        equal on every rank.  numpy arrays (host buffers) or 1-D torch CUDA tensors on the handle's device (device
+        buffers), float64 and contiguous.  Collective."""
+        nown = int(self.prec._lib.hymls_b200_owned_rows(self.prec._h, None, 0))
+        _check(self.prec._lib, nown)
+        return self._solve_local("ApplyInverseDist", self.prec._lib.hymls_b200_solve_dist, nown, b_local, T, x, seed,
+                                 history_cap)
+
+    def ApplyInverseMap(self, b_local, T=None, x=None, seed=43, history_cap=2048):
+        """ApplyInverseDist on the caller's rows declared with Preconditioner.SetRowMap, in that order."""
+        nlocal = getattr(self.prec, "_nlocal", None)
+        if nlocal is None:
+            raise HymlsError(-2, "ApplyInverseMap: call Preconditioner.SetRowMap first")
+        return self._solve_local("ApplyInverseMap", self.prec._lib.hymls_b200_solve_map, nlocal, b_local, T, x, seed,
+                                 history_cap)
+
+    def _solve_local(self, name, fn, nlocal, b_local, T, x, seed, history_cap):
+        P = self.prec
+        lib = P._lib
+        m = P.BorderSize()
+
+        def need(ok, what):
+            if not ok:
+                raise ValueError(name + ": " + what)
+
+        args = [("b_local", b_local, nlocal)] + ([("x", x, nlocal)] if x is not None else []) + \
+               ([("T", T, m)] if T is not None else [])
+        if isinstance(b_local, np.ndarray):
+            for what, a, ln in args:
+                need(isinstance(a, np.ndarray), "b_local is a numpy array, so %s must be one" % what)
+                need(a.dtype == np.float64, "%s must be float64" % what)
+                need(a.ndim == 1 and a.shape[0] == ln, "%s must be 1-D of length %d" % (what, ln))
+                need(a.flags.c_contiguous, "%s must be contiguous" % what)
+            xl = np.zeros(nlocal) if x is None else x
+            S = np.zeros(m)
+            where = HOST
+        else:
+            import torch
+            need(all(isinstance(a, torch.Tensor) for _, a, _ in args), "expected numpy arrays or torch tensors")
+            dev = _check(lib, lib.hymls_b200_get_device(P._h))
+            for what, a, ln in args:
+                need(a.is_cuda and a.device.index == dev, "%s must be a CUDA tensor on cuda:%d, the handle's device"
+                     % (what, dev))
+                need(a.dtype == torch.float64, "%s must be float64" % what)
+                need(a.dim() == 1 and a.shape[0] == ln, "%s must be 1-D of length %d" % (what, ln))
+                need(a.is_contiguous(), "%s must be contiguous" % what)
+            xl = torch.zeros_like(b_local) if x is None else x
+            S = torch.zeros(m, dtype=torch.float64, device=b_local.device)
+            where = DEVICE
+        p = lambda a: None if a is None else (a.ctypes.data if where == HOST else a.data_ptr())  # noqa: E731
+        info = _SolveInfo()
+        hist = np.zeros(history_cap)
+        _check(lib, fn(P._h, p(b_local), p(T) if m else None, p(xl), p(S) if m else None, where, seed, C.byref(info),
+                       hist.ctypes.data, history_cap))
+        self._keep_info(info, hist, history_cap)
+        return (xl, S) if m else xl
 
     def getNumIter(self):
         return self.num_iter

@@ -253,7 +253,23 @@ int hymls_b200_apply_matrix(hymls_b200_t* h, const double* x, double* y, int whe
 int hymls_b200_solve(hymls_b200_t* h, const double* b, double* x, int where, uint64_t seed,
                      hymls_b200_solve_info* info, double* hist, int cap) {
   HY_TRY
-  h->eng->solve(b, x, where, seed, info, hist, cap);
+  h->eng->solve(b, nullptr, x, nullptr, VecEnds::Replicated, where, seed, info, hist, cap);
+  return 0;
+  HY_CATCH
+}
+
+int hymls_b200_solve_dist(hymls_b200_t* h, const double* b_local, const double* T, double* x_local, double* S,
+                          int where, uint64_t seed, hymls_b200_solve_info* info, double* hist, int cap) {
+  HY_TRY
+  h->eng->solve(b_local, T, x_local, S, VecEnds::Owned, where, seed, info, hist, cap);
+  return 0;
+  HY_CATCH
+}
+
+int hymls_b200_solve_map(hymls_b200_t* h, const double* b_local, const double* T, double* x_local, double* S,
+                         int where, uint64_t seed, hymls_b200_solve_info* info, double* hist, int cap) {
+  HY_TRY
+  h->eng->solve(b_local, T, x_local, S, VecEnds::RowMap, where, seed, info, hist, cap);
   return 0;
   HY_CATCH
 }

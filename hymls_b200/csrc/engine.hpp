@@ -159,6 +159,10 @@ struct DistMatrixCache {
 
 // block-tridiagonal coarse factorization on BFS level sets (coarse.cu)
 struct KrylovLayout;  // the vector layout of one Krylov solve (krylov.cu)
+// where the caller's b, initial guess and x of a Krylov solve live: all n rows on every rank (hymls_b200_solve), the
+// rows of hymls_b200_owned_rows in that order (hymls_b200_solve_dist), or the caller's rows declared with setRowMap
+// (hymls_b200_solve_map)
+enum class VecEnds { Replicated, Owned, RowMap };
 
 struct CoarseBT {
   bool planned = false, active = false;
@@ -201,8 +205,10 @@ class Engine {
   void localRows(int64_t* r0, int64_t* r1) const;
   void applyInverseDist(const double* Bloc, double* Xloc, int where, const double* T = nullptr, double* S = nullptr);
   int64_t ownedRows(int64_t* rows, int64_t cap);
-  void solve(const double* b, double* x, int where, uint64_t seed, hymls_b200_solve_info* info, double* hist,
-             int histCap);
+  // T (border part of the right-hand side, nullptr: 0) and S (border part of the solution, nullptr: discarded) are
+  // replicated m-vectors on the same side as b and x; without a border they are not touched
+  void solve(const double* b, const double* T, double* x, double* S, VecEnds ends, int where, uint64_t seed,
+             hymls_b200_solve_info* info, double* hist, int histCap);
   void timeApply(int reps, double* msApply, double* msA11);
   void getStats(hymls_b200_stats* st);
   int64_t debugCopy(int level, const std::string& name, double* out, int64_t cap);
@@ -248,8 +254,8 @@ class Engine {
   void applyLevel0Dist(const double* B, double* X, const double* T = nullptr);  // with a border: S -> bS_
   void gatherOwned(const double* Xowned, double* Xfull);
   // Krylov solves on replicated vectors and on the owner distribution (krylov.cu)
-  KrylovLayout replicatedLayout(bool left, bool right);
-  KrylovLayout ownerLayout(bool left, bool right);
+  KrylovLayout replicatedLayout(bool left, bool right, VecEnds ends);
+  KrylovLayout ownerLayout(bool left, bool right, VecEnds ends);
   void applyDevice(const double* dB, double* dX, const double* dT = nullptr, double* dS = nullptr);
   bool applyDeviceMulti(const double* dB, int64_t ldb, double* dX, int64_t ldx, int nv);
   DevBuf<double> x1m_, y1m_;  // interior work vectors of the multi-column apply

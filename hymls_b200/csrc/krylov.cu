@@ -6,6 +6,8 @@
 //     owner path (HYMLS_B200_DIST=0, Number of Levels = 0).
 //   * owner: a rank holds the rows it owns (DistPlan, dist.cu), packed, followed by the border entries, which every
 //     rank keeps (bitwise equal); useDist() selects it.
+// Independently of the layout, the caller's b, x0 and x live on one of the VecEnds distributions; load and store
+// convert between the two at the ends of the solve, so the loop itself does not depend on the caller.
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -28,16 +30,20 @@ struct KrylovLayout {
   // free during a GMRES cycle
   std::function<void(const double* v, double* w)> step;
   std::function<const double*(const double* u)> expand;  // basis rows -> solution-side vector
-  std::function<void(const double* src, double* dst, cudaMemcpyKind kind)> load;   // b or x0 of the caller
+  // b or x0 of the caller, followed by the border entries T (nullptr: zeros)
+  std::function<void(const double* src, const double* T, double* dst, cudaMemcpyKind kind)> load;
   std::function<void(std::vector<double>& full)> keepOwn;  // a host vector of length n (+ border) -> this rank's part
-  std::function<void(const double* src, double* dst, cudaMemcpyKind kind)> store;  // x to the caller (replicated)
+  // x to the caller, and its border entries to S (nullptr: discarded)
+  std::function<void(const double* src, double* dst, double* S, cudaMemcpyKind kind)> store;
 };
 
 // Replicated vectors; the GMRES basis is row-sharded over the ranks: rank r keeps rows [r*chunk, (r+1)*chunk) of every
 // basis vector, so its Gram-Schmidt dots are local partial sums + one all-reduce of (k+1) doubles (the reference's
 // SumAll).  The preconditioner wants its argument replicated, so v_k is all-gathered before each ApplyInverse.
-KrylovLayout Engine::replicatedLayout(bool left, bool right) {
-  // With a border set the bordered system [K V; W' C] [x; s] = [b; 0] is solved on vectors of length n + m
+// Distributed ends: one all-gather of the owned rows builds the full b (with one rank the owned rows are all rows),
+// and each rank picks its rows out of x.
+KrylovLayout Engine::replicatedLayout(bool left, bool right, VecEnds ends) {
+  // With a border set the bordered system [K V; W' C] [x; s] = [b; T] is solved on vectors of length n + m
   // (HYMLS::BorderedSolver::ApplyInverse, src/HYMLS_BorderedSolver.cpp:159-219), preconditioned by the
   // bordered ApplyInverse.  ("Use Bordering" = true without a border is the plain solve with a warning there.)
   const int bm = borderM_;
@@ -95,13 +101,40 @@ KrylovLayout Engine::replicatedLayout(bool left, bool right) {
     }
   };
   L.expand = expand;
-  L.load = [=](const double* src, double* dst, cudaMemcpyKind kind) {
-    HY_CUDA(cudaMemcpyAsync(dst, src, nK * sizeof(double), kind, s));
-    if (bm) HY_CUDA(cudaMemsetAsync(dst + nK, 0, bm * sizeof(double), s));
+  DistPlan* D = P > 1 ? &levels_[0]->dist : nullptr;
+  RowMapPlan* R = &rowMap_;
+  const int64_t nOwn = D ? D->nOwn : nK;
+  if (ends == VecEnds::Owned && D) bufG_.alloc(nOwn);
+  L.load = [=](const double* src, const double* T, double* dst, cudaMemcpyKind kind) {
+    if (ends == VecEnds::Replicated || (ends == VecEnds::Owned && !D)) {
+      HY_CUDA(cudaMemcpyAsync(dst, src, nK * sizeof(double), kind, s));
+    } else {
+      if (ends == VecEnds::Owned) {
+        HY_CUDA(cudaMemcpyAsync(bufG_.p, src, nOwn * sizeof(double), kind, s));
+        scatterVec(bufG_.p, D->ownRows.p, dst, nOwn, s, &launches_);
+      } else {
+        if (R->nLocal) HY_CUDA(cudaMemcpyAsync(R->stage.p, src, R->nLocal * sizeof(double), kind, s));
+        haloExchange(R->toOwner, R->stage.p, dst, true);
+      }
+      if (D) gatherOwned(dst, dst);
+    }
+    if (!bm) return;
+    if (T) HY_CUDA(cudaMemcpyAsync(dst + nK, T, bm * sizeof(double), kind, s));
+    else HY_CUDA(cudaMemsetAsync(dst + nK, 0, bm * sizeof(double), s));
   };
   L.keepOwn = [](std::vector<double>&) {};
-  L.store = [=](const double* src, double* dst, cudaMemcpyKind kind) {
-    HY_CUDA(cudaMemcpyAsync(dst, src, nK * sizeof(double), kind, s));
+  L.store = [=](const double* src, double* dst, double* S, cudaMemcpyKind kind) {
+    if (ends == VecEnds::Replicated || (ends == VecEnds::Owned && !D)) {
+      HY_CUDA(cudaMemcpyAsync(dst, src, nK * sizeof(double), kind, s));
+    } else if (ends == VecEnds::Owned) {
+      packIdx(src, D->ownRows.p, bufG_.p, nOwn, s, &launches_);
+      HY_CUDA(cudaMemcpyAsync(dst, bufG_.p, nOwn * sizeof(double), kind, s));
+    } else {
+      double* cX = R->stage.p + std::max<int64_t>(R->nLocal, 1);
+      haloExchange(R->fromOwner, src, cX, true);
+      if (R->nLocal) HY_CUDA(cudaMemcpyAsync(dst, cX, R->nLocal * sizeof(double), kind, s));
+    }
+    if (bm && S) HY_CUDA(cudaMemcpyAsync(S, src + nK, bm * sizeof(double), kind, s));
   };
   return L;
 }
@@ -110,7 +143,10 @@ KrylovLayout Engine::replicatedLayout(bool left, bool right) {
 // the inner products); the basis lives in the same rows, so the loop contains no full-vector collective.  The
 // operator and the preconditioner work on global-length vectors with the owned entries valid: kS1_ (argument) and
 // kS2_ (result); the border adds one all-reduce of m doubles to the operator.
-KrylovLayout Engine::ownerLayout(bool left, bool right) {
+//
+// Ends: owned rows are copied straight into / out of the packed rows (no collective of length n); the caller's map
+// takes one grouped exchange each way (RowMapPlan, boundary.cu); replicated ends copy all n rows in and all-gather x.
+KrylovLayout Engine::ownerLayout(bool left, bool right, VecEnds ends) {
   Level* L0 = levels_[0].get();
   DistPlan* D = &L0->dist;
   buildMatrixHalo();
@@ -173,10 +209,22 @@ KrylovLayout Engine::ownerLayout(bool left, bool right) {
     }
   };
   L.expand = [](const double* u) { return u; };
-  L.load = [=](const double* src, double* dst, cudaMemcpyKind kind) {
-    HY_CUDA(cudaMemcpyAsync(gOut, src, n * sizeof(double), kind, s));
-    packIdx(gOut, D->ownRows.p, dst, nOwn, s, &launches_);
-    if (bm) HY_CUDA(cudaMemsetAsync(dst + nOwn, 0, bm * sizeof(double), s));
+  RowMapPlan* R = &rowMap_;
+  L.load = [=](const double* src, const double* T, double* dst, cudaMemcpyKind kind) {
+    if (ends == VecEnds::Owned) {
+      HY_CUDA(cudaMemcpyAsync(dst, src, nOwn * sizeof(double), kind, s));
+    } else {
+      if (ends == VecEnds::Replicated) {
+        HY_CUDA(cudaMemcpyAsync(gOut, src, n * sizeof(double), kind, s));
+      } else {
+        if (R->nLocal) HY_CUDA(cudaMemcpyAsync(R->stage.p, src, R->nLocal * sizeof(double), kind, s));
+        haloExchange(R->toOwner, R->stage.p, gOut, true);
+      }
+      packIdx(gOut, D->ownRows.p, dst, nOwn, s, &launches_);
+    }
+    if (!bm) return;
+    if (T) HY_CUDA(cudaMemcpyAsync(dst + nOwn, T, bm * sizeof(double), kind, s));
+    else HY_CUDA(cudaMemsetAsync(dst + nOwn, 0, bm * sizeof(double), s));
   };
   L.keepOwn = [=](std::vector<double>& full) {  // n + m host numbers -> owned rows + border entries
     std::vector<double> own(nOwn + bm);
@@ -184,19 +232,37 @@ KrylovLayout Engine::ownerLayout(bool left, bool right) {
     for (int j = 0; j < bm; ++j) own[nOwn + j] = full[n + j];
     full.swap(own);
   };
-  L.store = [=](const double* src, double* dst, cudaMemcpyKind kind) {  // replicated, like the single-GPU entry point
-    toGlobal(src, gIn);
-    gatherOwned(gIn, gOut);
-    HY_CUDA(cudaMemcpyAsync(dst, gOut, n * sizeof(double), kind, s));
+  L.store = [=](const double* src, double* dst, double* S, cudaMemcpyKind kind) {
+    if (ends == VecEnds::Owned) {
+      HY_CUDA(cudaMemcpyAsync(dst, src, nOwn * sizeof(double), kind, s));
+    } else if (ends == VecEnds::Replicated) {  // like the single-GPU entry point
+      toGlobal(src, gIn);
+      gatherOwned(gIn, gOut);
+      HY_CUDA(cudaMemcpyAsync(dst, gOut, n * sizeof(double), kind, s));
+    } else {
+      double* cX = R->stage.p + std::max<int64_t>(R->nLocal, 1);
+      toGlobal(src, gIn);
+      haloExchange(R->fromOwner, gIn, cX, true);
+      if (R->nLocal) HY_CUDA(cudaMemcpyAsync(dst, cX, R->nLocal * sizeof(double), kind, s));
+    }
+    if (bm && S) HY_CUDA(cudaMemcpyAsync(S, src + nOwn, bm * sizeof(double), kind, s));
   };
   return L;
 }
 
-void Engine::solve(const double* b, double* x, int where, uint64_t seed, hymls_b200_solve_info* info, double* hist,
-                   int histCap) {
+void Engine::solve(const double* b, const double* T, double* x, double* S, VecEnds ends, int where, uint64_t seed,
+                   hymls_b200_solve_info* info, double* hist, int histCap) {
   needDevice();
   needComm();
   if (!computed_) throw Error(HYMLS_B200_ERR_STATE, "The preconditioner has not yet been computed.");
+  if (ends != VecEnds::Replicated) {
+    const char* what = ends == VecEnds::Owned ? "solve_dist" : "solve_map";
+    if (!b || !x) throw Error(HYMLS_B200_ERR_ARG, std::string(what) + ": b_local and x_local are required");
+    if (ends == VecEnds::RowMap && !rowMap_.ready)
+      throw Error(HYMLS_B200_ERR_STATE, "solve_map: call hymls_b200_set_row_map first");
+    if (comm_.size() > 1 && !levels_[0]->dist.ready)
+      throw Error(HYMLS_B200_ERR_STATE, std::string(what) + ": no distributed plan (Number of Levels = 0?)");
+  }
   ParameterList& sol = params_.sublist("Solver");
   ParameterList& it = sol.sublist("Iterative Solver");
   if (sol.get("Use Deflation", false))
@@ -217,7 +283,7 @@ void Engine::solve(const double* b, double* x, int where, uint64_t seed, hymls_b
   if (borderM_ && !gmres) throw Error(HYMLS_B200_ERR_UNSUPPORTED, "bordered solves use GMRES");
   const int m = std::max(1, std::min(numBlocks, maxIters));
   const bool left = side == "Left", right = side == "Right";
-  const KrylovLayout L = useDist() ? ownerLayout(left, right) : replicatedLayout(left, right);
+  const KrylovLayout L = useDist() ? ownerLayout(left, right, ends) : replicatedLayout(left, right, ends);
   const int64_t n = L.len;
   cudaStream_t s = stream_;
 
@@ -233,7 +299,7 @@ void Engine::solve(const double* b, double* x, int where, uint64_t seed, hymls_b
   if (gmres) kV_.alloc((size_t)(m + 1) * L.rowLd);
   else kQ_.alloc(L.ld);
   const auto kind = where == HYMLS_B200_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-  L.load(b, kB_.p, kind);
+  L.load(b, T, kB_.p, kind);
   if (startVec == "Random") {
     // MatrixUtils::Random (src/HYMLS_MatrixUtils.cpp:961-1007): uniform in (-1,1); the reference's
     // Epetra_Util LCG stream is replaced by a documented 64-bit Mersenne Twister with `seed`.
@@ -246,7 +312,7 @@ void Engine::solve(const double* b, double* x, int where, uint64_t seed, hymls_b
   } else if (startVec == "Zero") {
     HY_CUDA(cudaMemsetAsync(kX_.p, 0, L.ld * sizeof(double), s));
   } else {
-    L.load(x, kX_.p, kind);
+    L.load(x, nullptr, kX_.p, kind);
   }
   // the ranks start the timed region together (a late rank would otherwise bill its delay to the others' first
   // collective)
@@ -440,8 +506,8 @@ void Engine::solve(const double* b, double* x, int where, uint64_t seed, hymls_b
   HY_CUDA(cudaStreamSynchronize(s));
   float ms = 0;
   HY_CUDA(cudaEventElapsedTime(&ms, ev0_, ev1_));
-  const double res = residual();  // explicit residual
-  L.store(kX_.p, x, where == HYMLS_B200_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost);
+  const double res = residual();  // explicit residual of [K V; W' C] [x; s] = [b; T]
+  L.store(kX_.p, x, S, where == HYMLS_B200_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost);
   HY_CUDA(cudaStreamSynchronize(s));
   if (info) {
     info->iterations = iters;

@@ -161,7 +161,7 @@ class B200Preconditioner : public Ifpack_Preconditioner, public BorderedOperator
   double Condest() const { return -1.0; }
   std::ostream& Print(std::ostream& os) const { return os << Label() << " (" << hymls_b200_version() << ")\n"; }
 
-  // HYMLS::Solver-side helpers when hymls_b200_solve replaces the Belos loop
+  // HYMLS::Solver-side helpers when the device Krylov solve replaces the Belos loop (see HYMLS_B200_Solver.hpp)
   int SetTolerance(double tol) { return hymls_b200_set_tolerance(h_, tol); }  // BaseSolver::SetTolerance
   std::string FinalParameterListXml() const {                                  // "Store Final Parameter List"
     std::string s((size_t)hymls_b200_get_parameters_xml(h_, nullptr, 0) + 1, '\0');

@@ -186,12 +186,37 @@ typedef struct {
   int iterations;
   int converged;
   double rel_residual;        /* last implicit relative residual */
-  double explicit_rel_residual; /* ||b - K x|| / ||b|| evaluated at the end */
+  double explicit_rel_residual; /* ||b - K x|| / ||b|| evaluated at the end ([b; T] and [K V; W' C] with a border) */
   double solve_seconds;       /* device time of the whole solve (CUDA events) */
   int history_len;
 } hymls_b200_solve_info;
 int hymls_b200_solve(hymls_b200_t* h, const double* b, double* x, int where, uint64_t random_seed,
                      hymls_b200_solve_info* info, double* resid_history, int history_cap);
+
+/*
+ * The same Krylov solve on distributed vectors (HYMLS::Solver::ApplyInverse / HYMLS::BorderedSolver::ApplyInverse on
+ * Epetra vectors of the matrix' row map), one right-hand side per call; collective.
+ * hymls_b200_solve_dist takes b_local and returns x_local on the rows of hymls_b200_owned_rows, in that order;
+ * hymls_b200_solve_map on the caller's rows declared with hymls_b200_set_row_map.  x_local holds the initial guess
+ * when Initial Vector = Previous and receives the solution.  With a border set (m = hymls_b200_border_size) the
+ * bordered system [K V; W' C] [x; s] = [b; T] is solved: T and S are replicated m-vectors, T == NULL means T = 0 and
+ * S == NULL discards s; S comes out bitwise equal on every rank.  Without a border m = 0 and T, S are neither read nor
+ * written.  `where` applies to b_local, x_local, T and S.  info->explicit_rel_residual is relative to ||[b; T]||.
+ * Initial Vector = Random draws the same stream as hymls_b200_solve (mt19937_64(random_seed), entry g for row g),
+ * so the solve does not depend on the distribution of the vectors.
+ * Only the ends differ from hymls_b200_solve: solve_dist copies b into this rank's rows and x out of them, with no
+ * collective of length n; solve_map adds one grouped exchange of the caller's rows each way (two with Previous for
+ * the initial guess).  Without the owner path (one rank, HYMLS_B200_DIST=0) one all-gather of the owned rows builds
+ * the full b and every rank picks its rows out of x.
+ * Refused: NULL b_local / x_local (HYMLS_B200_ERR_ARG), before Compute or solve_map before set_row_map
+ * (HYMLS_B200_ERR_STATE), CG with a border set (HYMLS_B200_ERR_UNSUPPORTED).
+ */
+int hymls_b200_solve_dist(hymls_b200_t* h, const double* b_local, const double* T, double* x_local, double* S,
+                          int where, uint64_t random_seed, hymls_b200_solve_info* info, double* resid_history,
+                          int history_cap);
+int hymls_b200_solve_map(hymls_b200_t* h, const double* b_local, const double* T, double* x_local, double* S,
+                         int where, uint64_t random_seed, hymls_b200_solve_info* info, double* resid_history,
+                         int history_cap);
 
 /* BaseSolver::SetTolerance (src/HYMLS_BaseSolver.cpp, used by NOX_Epetra_LinearSystem_Hymls.cpp:330-334 to
    override "Convergence Tolerance" per solve). */
