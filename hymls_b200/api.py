@@ -38,7 +38,8 @@ class _Stats(C.Structure):
                 ("kernel_launches", C.c_int64), ("device_bytes", C.c_double), ("sum_nsd_nb", C.c_double),
                 ("bytes_a11_full_pass", C.c_double), ("ms_a11_lead", C.c_double), ("interior_couplings", C.c_int64),
                 ("a11_split", C.c_int64), ("host_pipeline_chunks", C.c_int64), ("host_pipeline_state", C.c_int64),
-                ("collective_calls", C.c_int64), ("collective_bytes", C.c_int64), ("a11_entry_bytes", C.c_int64)]
+                ("collective_calls", C.c_int64), ("collective_bytes", C.c_int64), ("a11_entry_bytes", C.c_int64),
+                ("krylov_basis_bytes", C.c_int64)]
 
 
 def lib_path():

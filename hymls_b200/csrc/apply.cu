@@ -509,33 +509,68 @@ void householder(const int* uniqStart, int nuniq, const double* w, const double*
 // list, over rows[0..n).
 // The basis vectors are taken DOT_G at a time: one read of w[r] feeds DOT_G products with independent loads
 // in flight, and the block reduction is paid once per group instead of once per vector.
+// T is the element type of the basis: double, or float for the FP32 slots of "Krylov Basis Precision" = "Single"
+// (plain form only: no row list, no widx).  A float entry is widened to double as it is loaded; w, the products and the
+// sums are FP64.  VEC (float only; basis, ldv and w 16-byte aligned): a thread takes four rows at a time, one float4 per
+// basis vector, so eight 16-byte loads are in flight per lane where the FP64 kernel has eight 8-byte ones.
 static constexpr int DOT_G = 8;
+template <typename T, bool VEC = false>
 __global__ void __launch_bounds__(256)
-k_multi_dot(const double* __restrict__ V, int64_t ldv, int k, const double* __restrict__ w, int64_t n,
+k_multi_dot(const T* __restrict__ V, int64_t ldv, int k, const double* __restrict__ w, int64_t n,
             double* __restrict__ partial, const int* __restrict__ widx, const int* __restrict__ rows) {
   __shared__ double red[DOT_G][8];
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int i0 = 0; i0 < k; i0 += DOT_G) {
     const int ng = min(DOT_G, k - i0);
-    const double* __restrict__ v0 = V + (int64_t)i0 * ldv;
+    const T* __restrict__ v0 = V + (int64_t)i0 * ldv;
     double acc[DOT_G];
 #pragma unroll
     for (int g = 0; g < DOT_G; ++g) acc[g] = 0.0;
-    if (ng == DOT_G) {
-      for (int64_t i = (int64_t)blockIdx.x * blockDim.x + tid; i < n; i += stride) {
-        const int64_t r = rows ? (int64_t)rows[i] : i;
-        const double wv = widx ? w[widx[r]] : w[r];
+    if constexpr (sizeof(T) == sizeof(double)) {
+      if (ng == DOT_G) {
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + tid; i < n; i += stride) {
+          const int64_t r = rows ? (int64_t)rows[i] : i;
+          const double wv = widx ? w[widx[r]] : w[r];
 #pragma unroll
-        for (int g = 0; g < DOT_G; ++g) acc[g] += v0[(int64_t)g * ldv + r] * wv;
+          for (int g = 0; g < DOT_G; ++g) acc[g] += v0[(int64_t)g * ldv + r] * wv;
+        }
+      } else {
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + tid; i < n; i += stride) {
+          const int64_t r = rows ? (int64_t)rows[i] : i;
+          const double wv = widx ? w[widx[r]] : w[r];
+#pragma unroll
+          for (int g = 0; g < DOT_G; ++g)
+            if (g < ng) acc[g] += v0[(int64_t)g * ldv + r] * wv;
+        }
       }
+    } else if constexpr (VEC) {
+      const int64_t n4 = n >> 2, ld4 = ldv >> 2;
+      const float4* __restrict__ v4 = reinterpret_cast<const float4*>(v0);
+      for (int64_t i = (int64_t)blockIdx.x * blockDim.x + tid; i < n4; i += stride) {
+        const double2 wa = reinterpret_cast<const double2*>(w)[2 * i], wb = reinterpret_cast<const double2*>(w)[2 * i + 1];
+        float4 a[DOT_G];
+#pragma unroll
+        for (int g = 0; g < DOT_G; ++g) a[g] = g < ng ? v4[(int64_t)g * ld4 + i] : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+        for (int g = 0; g < DOT_G; ++g) {
+          acc[g] += (double)a[g].x * wa.x;
+          acc[g] += (double)a[g].y * wa.y;
+          acc[g] += (double)a[g].z * wb.x;
+          acc[g] += (double)a[g].w * wb.y;
+        }
+      }
+      if (blockIdx.x == 0 && tid == 0)  // the n % 4 tail rows
+        for (int64_t r = n4 << 2; r < n; ++r)
+#pragma unroll
+          for (int g = 0; g < DOT_G; ++g)
+            if (g < ng) acc[g] += (double)v0[(int64_t)g * ldv + r] * w[r];
     } else {
-      for (int64_t i = (int64_t)blockIdx.x * blockDim.x + tid; i < n; i += stride) {
-        const int64_t r = rows ? (int64_t)rows[i] : i;
-        const double wv = widx ? w[widx[r]] : w[r];
+      for (int64_t r = (int64_t)blockIdx.x * blockDim.x + tid; r < n; r += stride) {
+        const double wv = w[r];
 #pragma unroll
         for (int g = 0; g < DOT_G; ++g)
-          if (g < ng) acc[g] += v0[(int64_t)g * ldv + r] * wv;
+          if (g < ng) acc[g] += (double)v0[(int64_t)g * ldv + r] * wv;
       }
     }
 #pragma unroll
@@ -580,23 +615,81 @@ static const int DOT_BLOCKS = 592;  // 4 x 148 SMs
 void multiDot(const double* V, int64_t ldv, int k, const double* w, int64_t n, double* partial, double* h,
               int accumulate, cudaStream_t s, int64_t* launches, const int* widx, const int* rows) {
   if (k == 0) return;
-  k_multi_dot<<<DOT_BLOCKS, 256, 0, s>>>(V, ldv, k, w, n, partial, widx, rows);
+  k_multi_dot<double><<<DOT_BLOCKS, 256, 0, s>>>(V, ldv, k, w, n, partial, widx, rows);
+  k_reduce_partials<<<k, 256, 0, s>>>(partial, DOT_BLOCKS, k, h, accumulate);
+  *launches += 2;
+}
+// 16-byte loads of four floats need the basis, every basis vector and w (double2 pairs) on 16-byte boundaries
+static bool floatVec(const float* V, int64_t ldv, const double* w) {
+  return !(ldv & 3) && !(reinterpret_cast<uintptr_t>(V) & 15) && !(reinterpret_cast<uintptr_t>(w) & 15);
+}
+void multiDot(const float* V, int64_t ldv, int k, const double* w, int64_t n, double* partial, double* h,
+              int accumulate, cudaStream_t s, int64_t* launches) {
+  if (k == 0) return;
+  if (floatVec(V, ldv, w))
+    k_multi_dot<float, true><<<DOT_BLOCKS, 256, 0, s>>>(V, ldv, k, w, n, partial, nullptr, nullptr);
+  else k_multi_dot<float, false><<<DOT_BLOCKS, 256, 0, s>>>(V, ldv, k, w, n, partial, nullptr, nullptr);
   k_reduce_partials<<<k, 256, 0, s>>>(partial, DOT_BLOCKS, k, h, accumulate);
   *launches += 2;
 }
 int multiDotBlocks() { return DOT_BLOCKS; }
 
 // w += sign * sum_i h[i] V_i : coefficients in shared memory; a thread owns two adjacent rows (16-byte loads,
-// eight of them in flight) when the basis is 16-byte aligned, one row otherwise
-template <bool PAIR>
+// eight of them in flight) when the basis is 16-byte aligned, one row otherwise.
+// T = float (the FP32 slots of "Krylov Basis Precision" = "Single"): entries widened to double as they are loaded, FP64
+// products and sums; with PAIR a thread owns four adjacent rows (one float4 per basis vector, eight in flight).
+template <typename T, bool PAIR>
 __global__ void __launch_bounds__(256)
-k_multi_axpy(const double* __restrict__ V, int64_t ldv, int k, const double* __restrict__ h,
+k_multi_axpy(const T* __restrict__ V, int64_t ldv, int k, const double* __restrict__ h,
              double* __restrict__ w, int64_t n, double sign) {
   extern __shared__ double sh[];
   for (int i = threadIdx.x; i < k; i += blockDim.x) sh[i] = h[i];
   __syncthreads();
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  if (PAIR) {
+  if constexpr (sizeof(T) == sizeof(float) && PAIR) {
+    const int64_t n4 = n >> 2, ld4 = ldv >> 2;
+    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n4; r += stride) {
+      const float4* __restrict__ v = reinterpret_cast<const float4*>(V) + r;
+      double s0[4] = {0.0, 0.0, 0.0, 0.0}, s1[4] = {0.0, 0.0, 0.0, 0.0};  // two sets: 16 accumulator registers
+      auto add = [](double* acc, double c0, float4 a, double c1, float4 b) {
+        acc[0] += c0 * (double)a.x + c1 * (double)b.x;
+        acc[1] += c0 * (double)a.y + c1 * (double)b.y;
+        acc[2] += c0 * (double)a.z + c1 * (double)b.z;
+        acc[3] += c0 * (double)a.w + c1 * (double)b.w;
+      };
+      int i = 0;
+      for (; i + 8 <= k; i += 8) {
+        const float4 a0 = v[(int64_t)i * ld4], a1 = v[(int64_t)(i + 1) * ld4], a2 = v[(int64_t)(i + 2) * ld4],
+                     a3 = v[(int64_t)(i + 3) * ld4], a4 = v[(int64_t)(i + 4) * ld4], a5 = v[(int64_t)(i + 5) * ld4],
+                     a6 = v[(int64_t)(i + 6) * ld4], a7 = v[(int64_t)(i + 7) * ld4];
+        add(s0, sh[i], a0, sh[i + 4], a4);
+        add(s1, sh[i + 1], a1, sh[i + 5], a5);
+        add(s0, sh[i + 2], a2, sh[i + 6], a6);
+        add(s1, sh[i + 3], a3, sh[i + 7], a7);
+      }
+      for (; i < k; ++i) {
+        const float4 a0 = v[(int64_t)i * ld4];
+        s0[0] += sh[i] * (double)a0.x;
+        s0[1] += sh[i] * (double)a0.y;
+        s0[2] += sh[i] * (double)a0.z;
+        s0[3] += sh[i] * (double)a0.w;
+      }
+      double2* wp = reinterpret_cast<double2*>(w) + 2 * r;
+      double2 wa = wp[0], wb = wp[1];
+      wa.x += sign * (s0[0] + s1[0]);
+      wa.y += sign * (s0[1] + s1[1]);
+      wb.x += sign * (s0[2] + s1[2]);
+      wb.y += sign * (s0[3] + s1[3]);
+      wp[0] = wa;
+      wp[1] = wb;
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0)  // the n % 4 tail rows
+      for (int64_t r = n4 << 2; r < n; ++r) {
+        double s = 0.0;
+        for (int i = 0; i < k; ++i) s += sh[i] * (double)V[(int64_t)i * ldv + r];
+        w[r] += sign * s;
+      }
+  } else if constexpr (PAIR) {
     const int64_t n2 = n >> 1;
     for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n2; r += stride) {
       const double2* __restrict__ v = reinterpret_cast<const double2*>(V) + r;
@@ -635,7 +728,7 @@ k_multi_axpy(const double* __restrict__ V, int64_t ldv, int k, const double* __r
     }
   } else {
     for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += stride) {
-      const double* __restrict__ v = V + r;
+      const T* __restrict__ v = V + r;
       double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
       int i = 0;
       for (; i + 8 <= k; i += 8) {
@@ -647,19 +740,31 @@ k_multi_axpy(const double* __restrict__ V, int64_t ldv, int k, const double* __r
         s2 += sh[i + 2] * a2 + sh[i + 6] * a6;
         s3 += sh[i + 3] * a3 + sh[i + 7] * a7;
       }
-      for (; i < k; ++i) s0 += sh[i] * v[(int64_t)i * ldv];
+      for (; i < k; ++i) s0 += sh[i] * (double)v[(int64_t)i * ldv];
       w[r] += sign * ((s0 + s1) + (s2 + s3));
     }
   }
 }
+static void checkAxpyK(int k) {
+  if ((size_t)k * sizeof(double) > 48 * 1024)
+    throw Error(HYMLS_B200_ERR_UNSUPPORTED, "more than 6144 Krylov vectors in one orthogonalisation");
+}
 void multiAxpy(const double* V, int64_t ldv, int k, const double* h, double* w, int64_t n, double sign,
                cudaStream_t s, int64_t* launches) {
   if (k == 0 || n == 0) return;
-  if ((size_t)k * sizeof(double) > 48 * 1024)
-    throw Error(HYMLS_B200_ERR_UNSUPPORTED, "more than 6144 Krylov vectors in one orthogonalisation");
+  checkAxpyK(k);
   const bool pair = !(ldv & 1) && !(reinterpret_cast<uintptr_t>(V) & 15) && !(reinterpret_cast<uintptr_t>(w) & 15);
-  if (pair) k_multi_axpy<true><<<DOT_BLOCKS, 256, (size_t)k * sizeof(double), s>>>(V, ldv, k, h, w, n, sign);
-  else k_multi_axpy<false><<<DOT_BLOCKS, 256, (size_t)k * sizeof(double), s>>>(V, ldv, k, h, w, n, sign);
+  if (pair) k_multi_axpy<double, true><<<DOT_BLOCKS, 256, (size_t)k * sizeof(double), s>>>(V, ldv, k, h, w, n, sign);
+  else k_multi_axpy<double, false><<<DOT_BLOCKS, 256, (size_t)k * sizeof(double), s>>>(V, ldv, k, h, w, n, sign);
+  ++*launches;
+}
+void multiAxpy(const float* V, int64_t ldv, int k, const double* h, double* w, int64_t n, double sign,
+               cudaStream_t s, int64_t* launches) {
+  if (k == 0 || n == 0) return;
+  checkAxpyK(k);
+  if (floatVec(V, ldv, w))
+    k_multi_axpy<float, true><<<DOT_BLOCKS, 256, (size_t)k * sizeof(double), s>>>(V, ldv, k, h, w, n, sign);
+  else k_multi_axpy<float, false><<<DOT_BLOCKS, 256, (size_t)k * sizeof(double), s>>>(V, ldv, k, h, w, n, sign);
   ++*launches;
 }
 // y = a*x + b*y   (b == 0 : y = a*x, no read of y)
@@ -683,6 +788,24 @@ __global__ void k_scale_by_inv(const double* __restrict__ x, const double* __res
 void scaleByInvNorm(const double* x, const double* nrm2, double* y, int64_t n, cudaStream_t s, int64_t* launches) {
   if (n == 0) return;
   k_scale_by_inv<<<DOT_BLOCKS, 256, 0, s>>>(x, nrm2, y, n);
+  ++*launches;
+}
+// y = (float)(x * (1 / sqrt(*nrm2))), the product in FP64 rounded to nearest even (the next FP32 basis vector of
+// "Krylov Basis Precision" = "Single"); wide (optional) = y widened back to double, the exact vector stored in y
+__global__ void k_scale_narrow(const double* __restrict__ x, const double* __restrict__ nrm2, float* __restrict__ y,
+                               double* __restrict__ wide, int64_t n) {
+  const double inv = 1.0 / sqrt(*nrm2);
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += stride) {
+    const float f = __double2float_rn(x[r] * inv);
+    y[r] = f;
+    if (wide) wide[r] = (double)f;
+  }
+}
+void scaleByInvNormNarrow(const double* x, const double* nrm2, float* y, double* wide, int64_t n, cudaStream_t s,
+                          int64_t* launches) {
+  if (n == 0) return;
+  k_scale_narrow<<<DOT_BLOCKS, 256, 0, s>>>(x, nrm2, y, wide, n);
   ++*launches;
 }
 // y[i] = b[idx[i]] + t[i]

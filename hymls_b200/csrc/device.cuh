@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <atomic>
 #include <cstdint>
 #include <cstdio>
 #include <string>
@@ -20,6 +21,9 @@ namespace hymls {
                                                     " at " + __FILE__ + ":" + std::to_string(__LINE__)); \
   } while (0)
 
+// device memory held by the DevBuf and DeviceArena allocations of this process (hymls_b200_stats::device_bytes)
+extern std::atomic<int64_t> g_deviceBytes;
+
 // Bump allocator for the index arrays of one level.  A level holds ~100 immutable device arrays, sized once per
 // sparsity pattern; cudaMalloc costs 3-10 ms a call on a 180 GB device (measured: 7 small allocations = 68 ms), so
 // Initialize takes them from 256 MB slabs instead.  Memory goes back when the level is destroyed.
@@ -28,11 +32,13 @@ struct DeviceArena {
   std::vector<void*> slabs;
   char* cur = nullptr;
   size_t left = 0;
+  size_t held = 0;  // bytes of the slabs (counted in g_deviceBytes)
   explicit DeviceArena(size_t slab = (size_t)256 << 20, size_t direct = (size_t)64 << 20) : SLAB(slab), DIRECT(direct) {}
   DeviceArena(const DeviceArena&) = delete;
   DeviceArena& operator=(const DeviceArena&) = delete;
   ~DeviceArena() {
     for (void* p : slabs) cudaFree(p);
+    g_deviceBytes -= (int64_t)held;
   }
   void* take(size_t bytes) {
     bytes = (bytes + 255) & ~(size_t)255;
@@ -40,12 +46,16 @@ struct DeviceArena {
     if (bytes >= DIRECT) {  // large arrays get their own allocation (still owned by the arena)
       HY_CUDA(cudaMalloc(&p, bytes));
       slabs.push_back(p);
+      held += bytes;
+      g_deviceBytes += (int64_t)bytes;
       return p;
     }
     if (bytes > left) {
       const size_t slab = bytes > SLAB ? bytes : SLAB;
       HY_CUDA(cudaMalloc(&p, slab));
       slabs.push_back(p);
+      held += slab;
+      g_deviceBytes += (int64_t)slab;
       cur = (char*)p;
       left = slab;
     }
@@ -61,10 +71,13 @@ struct DeviceArena {
   }
   // a buffer that is re-allocated (grown) returns its memory: direct allocations are freed, slab pieces stay
   void giveBack(void* p, size_t bytes) {
-    if (((bytes + 255) & ~(size_t)255) < DIRECT) return;
+    bytes = (bytes + 255) & ~(size_t)255;
+    if (bytes < DIRECT) return;
     for (size_t k = 0; k < slabs.size(); ++k)
       if (slabs[k] == p) {
         cudaFree(p);
+        held -= bytes;
+        g_deviceBytes -= (int64_t)bytes;
         slabs.erase(slabs.begin() + k);
         return;
       }
@@ -89,8 +102,12 @@ struct DevBuf {
   DevBuf& operator=(const DevBuf&) = delete;
   ~DevBuf() { release(); }
   void release() {
-    if (p && owner) owner->giveBack(p, cap * sizeof(T));
-    else if (p) cudaFree(p);
+    if (p && owner) {
+      owner->giveBack(p, cap * sizeof(T));
+    } else if (p) {
+      cudaFree(p);
+      g_deviceBytes -= (int64_t)(cap * sizeof(T));
+    }
     p = nullptr;
     n = 0;
     cap = 0;
@@ -109,6 +126,7 @@ struct DevBuf {
       owner = g_arena;
     } else {
       HY_CUDA(cudaMalloc((void**)&p, count * sizeof(T)));
+      g_deviceBytes += (int64_t)(count * sizeof(T));
     }
   }
   void upload(const std::vector<T>& h, cudaStream_t s) {
@@ -132,7 +150,5 @@ struct PerDeviceLimit {
     return true;
   }
 };
-
-extern thread_local double g_devBytes;  // running total for statistics
 
 }  // namespace hymls

@@ -12,8 +12,8 @@
 
 namespace hymls {
 
-thread_local double g_devBytes = 0;
 thread_local DeviceArena* g_arena = nullptr;
+std::atomic<int64_t> g_deviceBytes{0};
 
 static const double SMALL_ENTRY = 1e-14;  // HYMLS_SMALL_ENTRY
 
@@ -82,6 +82,18 @@ void Engine::readParameters() {
     if (p != "Double" && p != "Single")
       throw Error(HYMLS_B200_ERR_ARG, "Subdomain Inverse Precision '" + p + "': valid values are 'Double' and 'Single'");
     singleInverses_ = p == "Single";
+  }
+  // extension: FP32 storage of the GMRES basis (DESIGN.md, Deviations); like the above, the default is not written
+  // back, and a list without a "Solver" sublist does not get one
+  singleBasis_ = false;
+  if (params_.isSublist("Solver") && params_.sublist("Solver").isParameter("Krylov Basis Precision")) {
+    ParameterList& sol = params_.sublist("Solver");
+    const std::string p = sol.get("Krylov Basis Precision", "Double");  // a value that is no string throws
+    if (p != "Double" && p != "Single")
+      throw Error(HYMLS_B200_ERR_ARG, "Krylov Basis Precision '" + p + "': valid values are 'Double' and 'Single'");
+    if (p == "Single" && sol.isParameter("Krylov Method") && sol.get("Krylov Method", "GMRES") == "CG")
+      throw Error(HYMLS_B200_ERR_ARG, "Krylov Basis Precision 'Single' applies to GMRES: CG keeps no basis");
+    singleBasis_ = p == "Single";
   }
   std::string method = prec.get("Partitioner", "Cartesian");
   if (method != "Cartesian" && method != "Skew Cartesian")
@@ -2335,6 +2347,8 @@ void Engine::getStats(hymls_b200_stats* st) {
   }
   st->collective_calls = comm_.calls();
   st->collective_bytes = comm_.bytes();
+  st->device_bytes = (double)g_deviceBytes.load();
+  st->krylov_basis_bytes = (int64_t)(kV_.cap * sizeof(double) + kVf_.cap * sizeof(float));
 }
 
 }  // namespace hymls

@@ -300,6 +300,11 @@ class Engine {
   // Krylov workspace
   DevBuf<double> kV_, kW_, kZ_, kH_, kPartial_, kX_, kB_, kR_, kQ_;
   DevBuf<double> kS1_, kS2_;  // scratch of the vector layouts
+  // "Krylov Basis Precision" = "Single": kV_ holds only v0 of a GMRES cycle, kVf_ the FP32 slots 1..m, and kGs_ the
+  // FP64 vector being orthogonalised followed by the widened slot that the next Arnoldi step reads
+  bool singleBasis_ = false;
+  DevBuf<float> kVf_;
+  DevBuf<double> kGs_;
   int kCap_ = 0;
   // statistics
   hymls_b200_stats stats_{};

@@ -170,12 +170,20 @@ void householder(const int* uniqStart, int nuniq, const double* w, const double*
 // (fixed reduction order, no atomics).
 void multiDot(const double* V, int64_t ldv, int k, const double* w, int64_t n, double* partial, double* h,
               int accumulate, cudaStream_t s, int64_t* launches, const int* widx = nullptr, const int* rows = nullptr);
+// the same over an FP32 basis (entries widened to double, FP64 products and sums), plain form
+void multiDot(const float* V, int64_t ldv, int k, const double* w, int64_t n, double* partial, double* h,
+              int accumulate, cudaStream_t s, int64_t* launches);
 int multiDotBlocks();
 
 void multiAxpy(const double* V, int64_t ldv, int k, const double* h, double* w, int64_t n, double sign,
                cudaStream_t s, int64_t* launches);
+void multiAxpy(const float* V, int64_t ldv, int k, const double* h, double* w, int64_t n, double sign,
+               cudaStream_t s, int64_t* launches);
 void axpby(double a, const double* x, double b, double* y, int64_t n, cudaStream_t s, int64_t* launches);
 void scaleByInvNorm(const double* x, const double* nrm2, double* y, int64_t n, cudaStream_t s, int64_t* launches);
+// y = (float)(x * (1 / sqrt(*nrm2))) (FP64 product, round to nearest even); wide (nullptr: not written) = (double)y
+void scaleByInvNormNarrow(const double* x, const double* nrm2, float* y, double* wide, int64_t n, cudaStream_t s,
+                          int64_t* launches);
 void setValue(double* x, int64_t idx, double v, cudaStream_t s, int64_t* launches);
 void csrToDense(const int64_t* ptr, const int* col, const double* val, double* D, int n, int np, cudaStream_t s,
                 int64_t* launches);

@@ -280,6 +280,7 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
   if (method != "GMRES" && method != "CG")
     throw Error(HYMLS_B200_ERR_ARG, "Krylov Method '" + method + "' not supported (GMRES, CG)");
   const bool gmres = method == "GMRES";
+  const bool single = gmres && singleBasis_;  // FP32 basis slots 1..m (readParameters refuses Single with CG)
   if (borderM_ && !gmres) throw Error(HYMLS_B200_ERR_UNSUPPORTED, "bordered solves use GMRES");
   const int m = std::max(1, std::min(numBlocks, maxIters));
   const bool left = side == "Left", right = side == "Right";
@@ -295,9 +296,20 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
   kH_.alloc(2 * m + 8);
   kPartial_.alloc((size_t)(m + 2) * multiDotBlocks());
   // the Krylov basis is workspace like the vectors above (grow-only, reused by later solves): a 40 GB cudaMalloc
-  // does not belong into the event-timed iteration
-  if (gmres) kV_.alloc((size_t)(m + 1) * L.rowLd);
-  else kQ_.alloc(L.ld);
+  // does not belong into the event-timed iteration.  Each basis precision releases the storage of the other, so
+  // switching a handle's mode frees that memory.
+  if (single) {
+    if (kV_.cap > (size_t)L.rowLd) kV_.release();
+    kV_.alloc(L.rowLd);
+    kVf_.alloc((size_t)m * L.rowLd);
+    kGs_.alloc(2 * (size_t)L.rowLd);
+  } else if (gmres) {
+    kVf_.release();
+    kGs_.release();
+    kV_.alloc((size_t)(m + 1) * L.rowLd);
+  } else {
+    kQ_.alloc(L.ld);
+  }
   const auto kind = where == HYMLS_B200_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
   L.load(b, T, kB_.p, kind);
   if (startVec == "Random") {
@@ -370,7 +382,18 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
     }
   } else {
     const int64_t ldV = L.rowLd, nloc = L.rows, nDot = L.dotRows;
-    HY_CUDA(cudaMemsetAsync(kV_.p, 0, (size_t)(m + 1) * ldV * sizeof(double), s));
+    HY_CUDA(cudaMemsetAsync(kV_.p, 0, kV_.bytes(), s));
+    if (single) {
+      HY_CUDA(cudaMemsetAsync(kVf_.p, 0, kVf_.bytes(), s));
+      HY_CUDA(cudaMemsetAsync(kGs_.p, 0, kGs_.bytes(), s));
+    }
+    // Single: v0 stays FP64 in kV_ (rounding it would leave beta 2^-24 of r0 that no cycle can remove); slot j of
+    // 1..m is FP32 at Vf + (j-1) ldV.  The Arnoldi step reads v0 or the widened slot vin, bitwise the vector that the
+    // update of x uses; w is an FP64 work vector, orthogonalised in FP64 against v0 and the widened slots.
+    const double* v0 = kV_.p;
+    float* Vf = kVf_.p;
+    double* wS = single ? kGs_.p : nullptr;
+    double* vin = single ? kGs_.p + ldV : nullptr;
     std::vector<double> H((size_t)(m + 1) * m, 0.0), cs(m), sn(m), g(m + 1), hbuf(2 * m + 8);
     double* dH1 = kH_.p;              // first Gram-Schmidt pass  (m+1)
     double* dH2 = kH_.p + (m + 1);    // second pass              (m+1)
@@ -408,8 +431,8 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
       g[0] = beta;
       int kDone = 0;
       for (int k = 0; k < m && iters < maxIters; ++k) {
-        double* vk = kV_.p + (size_t)k * ldV;
-        double* w = kV_.p + (size_t)(k + 1) * ldV;
+        const double* vk = !single ? kV_.p + (size_t)k * ldV : k == 0 ? v0 : vin;
+        double* w = single ? wS : kV_.p + (size_t)(k + 1) * ldV;
         const bool lapIt = verboseSolve && comm_.rank() == 0 && (k % 50) == 20;
         auto tl = std::chrono::steady_clock::now();
         auto lap = [&](const char* what) {
@@ -427,15 +450,25 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
         L.step(vk, w);
         lap("operator step");
         // two passes of classical Gram-Schmidt (Belos ICGS/DGKS), fused multi-dot + multi-axpy
-        multiDot(kV_.p, ldV, k + 1, w, nDot, kPartial_.p, dH1, 0, s, &launches_);
-        comm_.allReduceSum(dH1, (size_t)(k + 1), s);
-        multiAxpy(kV_.p, ldV, k + 1, dH1, w, nloc, -1.0, s, &launches_);
-        multiDot(kV_.p, ldV, k + 1, w, nDot, kPartial_.p, dH2, 0, s, &launches_);
-        comm_.allReduceSum(dH2, (size_t)(k + 1), s);
-        multiAxpy(kV_.p, ldV, k + 1, dH2, w, nloc, -1.0, s, &launches_);
+        for (double* dh : {dH1, dH2}) {
+          if (single) {  // h[0] against v0, h[1..k] against the FP32 slots 1..k
+            multiDot(v0, ldV, 1, w, nDot, kPartial_.p, dh, 0, s, &launches_);
+            multiDot(Vf, ldV, k, w, nDot, kPartial_.p, dh + 1, 0, s, &launches_);
+          } else {
+            multiDot(kV_.p, ldV, k + 1, w, nDot, kPartial_.p, dh, 0, s, &launches_);
+          }
+          comm_.allReduceSum(dh, (size_t)(k + 1), s);
+          if (single) {
+            multiAxpy(v0, ldV, 1, dh, w, nloc, -1.0, s, &launches_);
+            multiAxpy(Vf, ldV, k, dh + 1, w, nloc, -1.0, s, &launches_);
+          } else {
+            multiAxpy(kV_.p, ldV, k + 1, dh, w, nloc, -1.0, s, &launches_);
+          }
+        }
         multiDot(w, ldV, 1, w, nDot, kPartial_.p, dNrm, 0, s, &launches_);
         comm_.allReduceSum(dNrm, 1, s);
-        scaleByInvNorm(w, dNrm, w, nloc, s, &launches_);
+        if (single) scaleByInvNormNarrow(w, dNrm, Vf + (size_t)k * ldV, vin, nloc, s, &launches_);
+        else scaleByInvNorm(w, dNrm, w, nloc, s, &launches_);
         lap("CGS2 (4 sweeps, 3 allreduces)");
         HY_CUDA(cudaMemcpyAsync(hbuf.data(), kH_.p, (2 * m + 3) * sizeof(double), cudaMemcpyDeviceToHost, s));
         HY_CUDA(cudaStreamSynchronize(s));
@@ -476,7 +509,12 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
         }
         HY_CUDA(cudaMemcpyAsync(dH1, y.data(), kDone * sizeof(double), cudaMemcpyHostToDevice, s));
         HY_CUDA(cudaMemsetAsync(kZ_.p, 0, ldV * sizeof(double), s));
-        multiAxpy(kV_.p, ldV, kDone, dH1, kZ_.p, nloc, 1.0, s, &launches_);
+        if (single) {
+          multiAxpy(v0, ldV, 1, dH1, kZ_.p, nloc, 1.0, s, &launches_);
+          multiAxpy(Vf, ldV, kDone - 1, dH1 + 1, kZ_.p, nloc, 1.0, s, &launches_);
+        } else {
+          multiAxpy(kV_.p, ldV, kDone, dH1, kZ_.p, nloc, 1.0, s, &launches_);
+        }
         HY_CUDA(cudaStreamSynchronize(s));
         const double* upd = L.expand(kZ_.p);
         if (right) {
@@ -493,7 +531,10 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
         r = kZ_.p;
         beta = std::sqrt(dot(r, r));
       }
-      if (history.back() <= tol) {
+      // Single: the recurrence residual does not include the rounding of the basis, so the cycle counts as converged
+      // only when the residual recomputed in FP64 meets tol in the implicit criterion's own scaling as well
+      const bool fp64Met = !single || (left ? beta : trueRes) / impScale <= tol;
+      if (history.back() <= tol && fp64Met) {
         if (!explicitTest || trueRes / expScale <= tol) {
           converged = true;
           break;

@@ -181,6 +181,11 @@ int hymls_b200_apply_matrix(hymls_b200_t* h, const double* x, double* y, int whe
  * If a border is set the bordered system is solved (HYMLS::BorderedSolver) with right-hand side [b;0], on several
  * ranks on the owner distribution like the unbordered system (the m border entries are replicated on every rank).
  * resid_history (may be NULL) receives up to history_cap relative implicit residuals, iteration 0 first.
+ * "Krylov Basis Precision" ("Double", the default, or "Single"; GMRES only) stores the basis vectors after the first
+ * of each cycle in FP32, with all arithmetic in FP64: half the basis memory and half the bytes of the
+ * orthogonalisation, but different iterates and possibly more iterations.  A Single cycle counts as converged only
+ * when the residual recomputed in FP64 also meets the tolerance in the implicit scaling, so info->converged = 1 always
+ * means that the FP64 residual met it.
  */
 typedef struct {
   int iterations;
@@ -256,7 +261,7 @@ typedef struct {
                                    a11_entry_bytes * sum (n_sd^2 + n_sd * nb_sd), full second solve + leading rows of
                                    the first */
   int64_t kernel_launches;      /* launches issued by this handle so far */
-  double device_bytes;          /* device memory held */
+  double device_bytes;          /* device memory held by the library's buffers in this process (all handles) */
   double sum_nsd_nb;            /* sum n_sd * nb_sd (level 0): nb_sd = interior nodes that separator rows couple to;
                                    the first subdomain solve of ApplyInverse needs only these rows of A11^-1 */
   double bytes_a11_full_pass;   /* this rank's a11_entry_bytes * sum n_sd^2: one full pass over its level-0 inverses */
@@ -283,6 +288,12 @@ typedef struct {
   int64_t a11_entry_bytes;      /* bytes per stored entry of the subdomain inverses A11^-1 that ApplyInverse streams: 8, or 4
                                    with "Subdomain Inverse Precision" = "Single" (FP32 storage, FP64 arithmetic).
                                    bytes_a11_level0, bytes_a11_full_pass and the A11 term of bytes_apply count this many */
+  int64_t krylov_basis_bytes;   /* bytes of GMRES basis storage the handle holds, 0 before its first GMRES solve.  With m =
+                                   Num Blocks (at most Maximum Iterations) and rowLd the basis rows of this rank (n, n + border
+                                   entries, or n / ranks rounded up; the owned rows + border rounded up to 8 on the owner
+                                   distribution): 8 (m + 1) rowLd with "Krylov Basis Precision" = "Double", 4 m rowLd + 8 rowLd
+                                   (FP32 slots 1..m, FP64 first vector) with "Single".  Storage is grow-only within one mode:
+                                   the largest m so far counts; a solve in the other mode releases it */
 } hymls_b200_stats;
 int hymls_b200_get_stats(hymls_b200_t* h, hymls_b200_stats* st);
 
