@@ -39,7 +39,7 @@ class _Stats(C.Structure):
                 ("bytes_a11_full_pass", C.c_double), ("ms_a11_lead", C.c_double), ("interior_couplings", C.c_int64),
                 ("a11_split", C.c_int64), ("host_pipeline_chunks", C.c_int64), ("host_pipeline_state", C.c_int64),
                 ("collective_calls", C.c_int64), ("collective_bytes", C.c_int64), ("a11_entry_bytes", C.c_int64),
-                ("krylov_basis_bytes", C.c_int64)]
+                ("krylov_basis_bytes", C.c_int64), ("krylov_recycle_dim", C.c_int64)]
 
 
 def lib_path():

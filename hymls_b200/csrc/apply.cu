@@ -767,6 +767,143 @@ void multiAxpy(const float* V, int64_t ldv, int k, const double* h, double* w, i
   else k_multi_axpy<float, false><<<DOT_BLOCKS, 256, (size_t)k * sizeof(double), s>>>(V, ldv, k, h, w, n, sign);
   ++*launches;
 }
+// ---------------------------------------------------------------------------------------------
+// restart phase of GCRO-DR: many basis vectors against a few others, each basis read once
+// ---------------------------------------------------------------------------------------------
+// H[j * ldh + i] = X_i' Y_j for i < nx (at most BD_X per launch), j < ny (at most 32 per launch).  A block takes tiles
+// of BD_TILE rows: the tile of Y goes to shared memory (row-major, lane j reads column j), warp w owns the vectors
+// i = w + 8 q, q < BD_Q; each lane loads four rows of X_i, broadcasts them by shuffles and accumulates X_i' Y_lane
+// over the tile.  Every lane keeps BD_Q sums over all its block's tiles (fixed order), and the per-block partials are
+// reduced in block order (deterministic, no atomics).
+static constexpr int BD_TILE = 128, BD_Q = 16, BD_X = 8 * BD_Q, BD_BLOCKS = 296;
+__global__ void __launch_bounds__(256, 2)
+k_block_dot(const double* __restrict__ X, int64_t ldx, int nx, const double* __restrict__ Y, int64_t ldy, int ny,
+            int64_t n, double* __restrict__ partial) {
+  __shared__ double ys[BD_TILE][33];  // row padded to 33: the staging stores of one warp hit different banks
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  double acc[BD_Q];
+#pragma unroll
+  for (int q = 0; q < BD_Q; ++q) acc[q] = 0.0;
+  for (int64_t t0 = (int64_t)blockIdx.x * BD_TILE; t0 < n; t0 += (int64_t)gridDim.x * BD_TILE) {
+    for (int idx = tid; idx < BD_TILE * ny; idx += blockDim.x) {  // lanes >= ny compute sums that are never stored
+      const int j = idx / BD_TILE, r = idx % BD_TILE;
+      ys[r][j] = t0 + r < n ? Y[(int64_t)j * ldy + t0 + r] : 0.0;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int q = 0; q < BD_Q; ++q) {
+      const int i = wid + 8 * q;
+      if (i < nx) {  // warp-uniform
+        const double* __restrict__ xi = X + (int64_t)i * ldx + t0;
+        double xs[BD_TILE / 32];
+#pragma unroll
+        for (int s = 0; s < BD_TILE / 32; ++s) xs[s] = t0 + lane + 32 * s < n ? xi[lane + 32 * s] : 0.0;
+#pragma unroll
+        for (int s = 0; s < BD_TILE / 32; ++s)
+#pragma unroll 8
+          for (int src = 0; src < 32; ++src)
+            acc[q] += __shfl_sync(0xffffffffu, xs[s], src) * ys[32 * s + src][lane];
+      }
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int q = 0; q < BD_Q; ++q) {
+    const int i = wid + 8 * q;
+    if (i < nx && lane < ny) partial[((int64_t)lane * nx + i) * gridDim.x + blockIdx.x] = acc[q];
+  }
+}
+// H[j * ldh + i] = sum_b partial[(j * nx + i) * nblk + b]  (fixed order)
+__global__ void k_reduce_block_dot(const double* __restrict__ partial, int nblk, int nx, double* __restrict__ H,
+                                   int64_t ldh) {
+  const int idx = blockIdx.x, i = idx % nx, j = idx / nx;
+  __shared__ double red[32];
+  double s = 0.0;
+  for (int b = threadIdx.x; b < nblk; b += blockDim.x) s += partial[(int64_t)idx * nblk + b];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) red[wid] = s;
+  __syncthreads();
+  if (wid == 0) {
+    s = lane < (blockDim.x >> 5) ? red[lane] : 0.0;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) H[(int64_t)j * ldh + i] = s;
+  }
+}
+size_t blockDotPartial() { return (size_t)BD_X * 32 * BD_BLOCKS; }
+void blockDot(const double* X, int64_t ldx, int nx, const double* Y, int64_t ldy, int ny, int64_t n, double* partial,
+              double* H, int64_t ldh, cudaStream_t s, int64_t* launches) {
+  for (int j0 = 0; j0 < ny; j0 += 32)
+    for (int i0 = 0; i0 < nx; i0 += BD_X) {
+      const int px = std::min(BD_X, nx - i0), py = std::min(32, ny - j0);
+      k_block_dot<<<BD_BLOCKS, 256, 0, s>>>(X + (int64_t)i0 * ldx, ldx, px, Y + (int64_t)j0 * ldy, ldy, py, n,
+                                            partial);
+      k_reduce_block_dot<<<px * py, 256, 0, s>>>(partial, BD_BLOCKS, px, H + (int64_t)j0 * ldh + i0, ldh);
+      *launches += 2;
+    }
+}
+
+// Y_j (+)= sum_i X_i coef[j * ldc + i] for i < nx (at most CB_X per launch), j < ny (at most NY): the coefficients in
+// shared memory, a thread keeps the NY sums of one row in registers, so X is read once per launch.
+static constexpr int CB_X = 128;
+template <int NY>
+__global__ void __launch_bounds__(256)
+k_combine(const double* __restrict__ X, int64_t ldx, int nx, const double* __restrict__ coef, int64_t ldc,
+          double* __restrict__ Y, int64_t ldy, int ny, int64_t n, int accumulate) {
+  __shared__ __align__(16) double cs[CB_X * NY];  // read as double2
+  for (int idx = threadIdx.x; idx < nx * NY; idx += blockDim.x) {
+    const int i = idx / NY, j = idx % NY;
+    cs[idx] = j < ny ? coef[(int64_t)j * ldc + i] : 0.0;
+  }
+  __syncthreads();
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += stride) {
+    double acc[NY];
+#pragma unroll
+    for (int j = 0; j < NY; ++j) acc[j] = 0.0;
+#pragma unroll 4
+    for (int i = 0; i < nx; ++i) {
+      const double x = X[(int64_t)i * ldx + r];
+      const double2* c2 = reinterpret_cast<const double2*>(cs + i * NY);
+#pragma unroll
+      for (int j = 0; j < NY / 2; ++j) {
+        const double2 c = c2[j];
+        acc[2 * j] += x * c.x;
+        acc[2 * j + 1] += x * c.y;
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < NY; ++j)
+      if (j < ny) {
+        double* y = Y + (int64_t)j * ldy + r;
+        *y = accumulate ? *y + acc[j] : acc[j];
+      }
+  }
+}
+void combine(const double* X, int64_t ldx, int nx, const double* coef, int64_t ldc, double* Y, int64_t ldy, int ny,
+             int64_t n, int accumulate, cudaStream_t s, int64_t* launches) {
+  if (n == 0 || ny == 0) return;
+  for (int j0 = 0; j0 < ny; j0 += 32) {
+    const int py = std::min(32, ny - j0);
+    double* Yj = Y + (int64_t)j0 * ldy;
+    if (nx == 0 && !accumulate) {
+      for (int j = 0; j < py; ++j) HY_CUDA(cudaMemsetAsync(Yj + (int64_t)j * ldy, 0, n * sizeof(double), s));
+      continue;
+    }
+    for (int i0 = 0; i0 < nx; i0 += CB_X) {
+      const int px = std::min(CB_X, nx - i0), acc = accumulate || i0 > 0;
+      const double* Xi = X + (int64_t)i0 * ldx;
+      const double* ci = coef + (int64_t)j0 * ldc + i0;
+      if (py <= 8) k_combine<8><<<DOT_BLOCKS, 256, 0, s>>>(Xi, ldx, px, ci, ldc, Yj, ldy, py, n, acc);
+      else if (py <= 16) k_combine<16><<<DOT_BLOCKS, 256, 0, s>>>(Xi, ldx, px, ci, ldc, Yj, ldy, py, n, acc);
+      else k_combine<32><<<DOT_BLOCKS, 256, 0, s>>>(Xi, ldx, px, ci, ldc, Yj, ldy, py, n, acc);
+      ++*launches;
+    }
+  }
+}
+
 // y = a*x + b*y   (b == 0 : y = a*x, no read of y)
 __global__ void k_axpby(double a, const double* __restrict__ x, double b, double* __restrict__ y, int64_t n) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;

@@ -95,6 +95,27 @@ void Engine::readParameters() {
       throw Error(HYMLS_B200_ERR_ARG, "Krylov Basis Precision 'Single' applies to GMRES: CG keeps no basis");
     singleBasis_ = p == "Single";
   }
+  // extension: GCRO-DR ("Krylov Method" = "GCRODR", DESIGN.md §5 item 12).  Only a GCRODR list is checked here, and
+  // nothing is written back: "Num Recycled Blocks" and its default are read by a GCRODR solve
+  if (params_.isSublist("Solver")) {
+    ParameterList& sol = params_.sublist("Solver");
+    const bool gcrodr = sol.isParameter("Krylov Method") && sol.kindOf("Krylov Method") == ParameterList::STRING &&
+                        sol.get("Krylov Method", "GMRES") == "GCRODR";
+    if (gcrodr && singleBasis_)
+      throw Error(HYMLS_B200_ERR_ARG, "Krylov Basis Precision 'Single' is not supported with GCRODR");
+    if (gcrodr && sol.isSublist("Iterative Solver")) {
+      ParameterList& it = sol.sublist("Iterative Solver");
+      if (it.isParameter("Num Recycled Blocks")) {
+        if (it.kindOf("Num Recycled Blocks") != ParameterList::INT)
+          throw Error(HYMLS_B200_ERR_ARG, "Num Recycled Blocks must be an integer");
+        const int k = it.get("Num Recycled Blocks", 5);
+        if (k < 1) throw Error(HYMLS_B200_ERR_ARG, "Num Recycled Blocks must be at least 1");
+        if (it.isParameter("Num Blocks") && it.kindOf("Num Blocks") == ParameterList::INT &&
+            k >= it.get("Num Blocks", 300))
+          throw Error(HYMLS_B200_ERR_ARG, "Num Recycled Blocks must be less than Num Blocks");
+      }
+    }
+  }
   std::string method = prec.get("Partitioner", "Cartesian");
   if (method != "Cartesian" && method != "Skew Cartesian")
     throw Error(HYMLS_B200_ERR_ARG, "Partitioner '" + method + "': Up to now we only support Cartesian partitioning");
@@ -118,6 +139,7 @@ void Engine::setParameters(const std::string& xml) {
     readParameters();
     throw;
   }
+  recDim_ = 0;  // a new list drops the recycled GCRO-DR space
   initialized_ = false;
   computed_ = false;
 }
@@ -323,6 +345,7 @@ GemvArgs BatchedInverse::args() const {
 // ---------------------------------------------------------------------------------------------
 void Engine::initialize() {
   if (!haveMatrix_) throw Error(HYMLS_B200_ERR_STATE, "Initialize: no matrix set");
+  recDim_ = 0;
   auto t0 = std::chrono::steady_clock::now();
   ParameterList levelParams = params_.deepCopy();
   levels_.resize(1);
@@ -886,6 +909,7 @@ void Engine::compute() {
   needDevice();
   needComm();
   computed_ = false;  // a Compute that throws must not leave half-updated factors marked usable
+  ++opEpoch_;         // a recycled GCRO-DR space rebuilds C = A U at the next solve
   if (!initialized_) initialize();  // "I'll do it for you", Preconditioner.cpp:403-409
   HY_CUDA(cudaEventRecord(ev0_, stream_));
   info_.alloc(1);
@@ -2348,7 +2372,8 @@ void Engine::getStats(hymls_b200_stats* st) {
   st->collective_calls = comm_.calls();
   st->collective_bytes = comm_.bytes();
   st->device_bytes = (double)g_deviceBytes.load();
-  st->krylov_basis_bytes = (int64_t)(kV_.cap * sizeof(double) + kVf_.cap * sizeof(float));
+  st->krylov_basis_bytes = (int64_t)((kV_.cap + kRec_.cap) * sizeof(double) + kVf_.cap * sizeof(float));
+  st->krylov_recycle_dim = recDim_;
 }
 
 }  // namespace hymls

@@ -256,6 +256,15 @@ class Engine {
   // Krylov solves on replicated vectors and on the owner distribution (krylov.cu)
   KrylovLayout replicatedLayout(bool left, bool right, VecEnds ends);
   KrylovLayout ownerLayout(bool left, bool right, VecEnds ends);
+  // GCRO-DR pieces of the Krylov driver (krylov.cu)
+  std::vector<double> crossProducts(const KrylovLayout& L, const double* X, int nx, const double* Y, int ny);
+  void recycleNorms(const KrylovLayout& L, int K1);
+  int rebuildRecycled(const KrylovLayout& L, int K1);
+  void recycleProject(const KrylovLayout& L, int K1, int kc, const double* r, bool right);
+  bool cycleStart(const KrylovLayout& L, double* base, int kc, const double* r, double* g, double* H, double* cs,
+                  double* sn, int m);
+  int recycleUpdate(const KrylovLayout& L, int K1, int recK, double* base, int kc, int kDone,
+                    const std::vector<double>& G, int m);
   void applyDevice(const double* dB, double* dX, const double* dT = nullptr, double* dS = nullptr);
   bool applyDeviceMulti(const double* dB, int64_t ldb, double* dX, int64_t ldx, int nv);
   DevBuf<double> x1m_, y1m_;  // interior work vectors of the multi-column apply
@@ -306,6 +315,17 @@ class Engine {
   DevBuf<float> kVf_;
   DevBuf<double> kGs_;
   int kCap_ = 0;
+  // GCRO-DR ("Krylov Method" = "GCRODR", krylov.cu).  The recycled space belongs to the handle and persists across
+  // solves: C (recDim_ columns, C' C = I) in the slots just before the Arnoldi vectors in kV_, U in kRec_ with
+  // A^ U = C for the operator A^ of the Krylov layout.  kRec_ holds two blocks of recCap_ columns, U and the scratch of
+  // the restart (recU_: index of U's block).  Dropped by Initialize, SetParameters and any change of the layout rows
+  // or border size; Compute bumps opEpoch_, and a solve whose recEpoch_ differs rebuilds C from U.
+  int recDim_ = 0, recCap_ = 0, recU_ = 0;
+  uint64_t opEpoch_ = 0, recEpoch_ = 0;
+  int64_t recRows_ = -1, recLd_ = -1, recRow0_ = -1;
+  int recBorder_ = -1, recM_ = -1;
+  std::vector<double> recD_;          // 1 / ||u_i||: the scaling of U inside the cycle (Parks et al., D_k)
+  DevBuf<double> kRec_, kSmall_, kPartialB_;
   // statistics
   hymls_b200_stats stats_{};
   int64_t launches_ = 0;

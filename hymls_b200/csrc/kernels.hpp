@@ -179,6 +179,14 @@ void multiAxpy(const double* V, int64_t ldv, int k, const double* h, double* w, 
                cudaStream_t s, int64_t* launches);
 void multiAxpy(const float* V, int64_t ldv, int k, const double* h, double* w, int64_t n, double sign,
                cudaStream_t s, int64_t* launches);
+// restart phase of GCRO-DR (deterministic, each X read once per 128 of its vectors and 32 of Y):
+// H[j * ldh + i] = X_i' Y_j over rows [0, n), i < nx, j < ny; partial: blockDotPartial() doubles
+void blockDot(const double* X, int64_t ldx, int nx, const double* Y, int64_t ldy, int ny, int64_t n, double* partial,
+              double* H, int64_t ldh, cudaStream_t s, int64_t* launches);
+size_t blockDotPartial();
+// Y_j (+)= sum_{i < nx} X_i coef[j * ldc + i] for j < ny, rows [0, n) (coef on the device, column major)
+void combine(const double* X, int64_t ldx, int nx, const double* coef, int64_t ldc, double* Y, int64_t ldy, int ny,
+             int64_t n, int accumulate, cudaStream_t s, int64_t* launches);
 void axpby(double a, const double* x, double b, double* y, int64_t n, cudaStream_t s, int64_t* launches);
 void scaleByInvNorm(const double* x, const double* nrm2, double* y, int64_t n, cudaStream_t s, int64_t* launches);
 // y = (float)(x * (1 / sqrt(*nrm2))) (FP64 product, round to nearest even); wide (nullptr: not written) = (double)y

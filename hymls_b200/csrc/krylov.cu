@@ -14,6 +14,7 @@
 #include <functional>
 #include <random>
 
+#include "dense_eig.hpp"
 #include "engine.hpp"
 
 namespace hymls {
@@ -250,6 +251,214 @@ KrylovLayout Engine::ownerLayout(bool left, bool right, VecEnds ends) {
   return L;
 }
 
+// ---- GCRO-DR (Parks, de Sturler, Mackey, Johnson, Maiti, SIAM J. Sci. Comput. 28(5), 2006, Algorithm 2) ----
+// The recycled space: U in kRec_ (block recU_), C = A^ U with C' C = I in the recDim_ slots before the Arnoldi vectors,
+// A^ = L.step.  Inside a cycle U enters scaled, Utilde = U D with D = diag(1 / ||u_i||) (recD_), so the first kc
+// columns of Ghat are D.  The small matrices are formed on every rank from all-reduced partial sums and handled by the
+// host routines of dense_eig.cpp, so every rank makes the same choices.
+
+// upper triangular inverse of R (n x n, column major)
+static std::vector<double> upperInverse(const std::vector<double>& R, int n) {
+  std::vector<double> X((size_t)n * n, 0.0);
+  for (int j = 0; j < n; ++j) {
+    X[(size_t)j * n + j] = 1.0 / R[(size_t)j * n + j];
+    for (int i = j - 1; i >= 0; --i) {
+      double t = 0.0;
+      for (int l = i + 1; l <= j; ++l) t += R[(size_t)l * n + i] * X[(size_t)j * n + l];
+      X[(size_t)j * n + i] = -t / R[(size_t)i * n + i];
+    }
+  }
+  return X;
+}
+
+// H = X' Y (nx x ny, column major) over this layout's rows, all-reduced, on the host
+std::vector<double> Engine::crossProducts(const KrylovLayout& L, const double* X, int nx, const double* Y, int ny) {
+  cudaStream_t s = stream_;
+  blockDot(X, L.rowLd, nx, Y, L.rowLd, ny, L.dotRows, kPartialB_.p, kSmall_.p, nx, s, &launches_);
+  comm_.allReduceSum(kSmall_.p, (size_t)nx * ny, s);
+  std::vector<double> h((size_t)nx * ny);
+  HY_CUDA(cudaMemcpyAsync(h.data(), kSmall_.p, h.size() * sizeof(double), cudaMemcpyDeviceToHost, s));
+  HY_CUDA(cudaStreamSynchronize(s));
+  return h;
+}
+
+void Engine::recycleNorms(const KrylovLayout& L, int K1) {
+  cudaStream_t s = stream_;
+  const double* U = kRec_.p + (size_t)recU_ * K1 * L.rowLd;
+  for (int i = 0; i < recDim_; ++i) {  // ||u_i||^2 into kSmall_[i]
+    const double* u = U + (size_t)i * L.rowLd;
+    multiDot(u, L.rowLd, 1, u, L.dotRows, kPartial_.p, kSmall_.p + i, 0, s, &launches_);
+  }
+  comm_.allReduceSum(kSmall_.p, (size_t)recDim_, s);
+  std::vector<double> g(recDim_);
+  HY_CUDA(cudaMemcpyAsync(g.data(), kSmall_.p, recDim_ * sizeof(double), cudaMemcpyDeviceToHost, s));
+  HY_CUDA(cudaStreamSynchronize(s));
+  recD_.assign(recDim_, 0.0);
+  for (int i = 0; i < recDim_; ++i) recD_[i] = 1.0 / std::sqrt(g[i]);
+}
+
+// C = A^ U after a Compute, then the thin QR C = Q R by two Cholesky-QR passes: C <- Q, U <- U R^-1.  Returns the
+// number of recycled columns kept (0: C was numerically rank deficient and the space is dropped).
+int Engine::rebuildRecycled(const KrylovLayout& L, int K1) {
+  cudaStream_t s = stream_;
+  const int kc = recDim_;
+  const int64_t ldV = L.rowLd;
+  double* Cb = kV_.p + (size_t)(K1 - kc) * ldV;
+  for (int i = 0; i < kc; ++i) L.step(kRec_.p + ((size_t)recU_ * K1 + i) * ldV, Cb + (size_t)i * ldV);
+  for (int pass = 0; pass < 2; ++pass) {
+    std::vector<double> g = crossProducts(L, Cb, kc, Cb, kc);
+    if (hy_cholesky(kc, g.data())) {
+      recDim_ = 0;
+      return 0;
+    }
+    std::vector<double> R((size_t)kc * kc);  // R = L'
+    for (int j = 0; j < kc; ++j)
+      for (int i = 0; i < kc; ++i) R[(size_t)j * kc + i] = g[(size_t)i * kc + j];
+    const std::vector<double> Ri = upperInverse(R, kc);
+    HY_CUDA(cudaMemcpyAsync(kSmall_.p, Ri.data(), Ri.size() * sizeof(double), cudaMemcpyHostToDevice, s));
+    double* U = kRec_.p + (size_t)recU_ * K1 * ldV;
+    double* scratch = kRec_.p + (size_t)(1 - recU_) * K1 * ldV;
+    combine(Cb, ldV, kc, kSmall_.p, kc, scratch, ldV, kc, L.rows, 0, s, &launches_);
+    HY_CUDA(cudaMemcpyAsync(Cb, scratch, (size_t)kc * ldV * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    combine(U, ldV, kc, kSmall_.p, kc, scratch, ldV, kc, L.rows, 0, s, &launches_);
+    recU_ = 1 - recU_;
+    HY_CUDA(cudaStreamSynchronize(s));  // Ri is pageable host memory
+  }
+  recEpoch_ = opEpoch_;
+  recycleNorms(L, K1);
+  return kc;
+}
+
+// x += [M^-1] U C' r (r: the residual the Krylov space is built on, b - A x or M^-1 (b - A x))
+void Engine::recycleProject(const KrylovLayout& L, int K1, int kc, const double* r, bool right) {
+  cudaStream_t s = stream_;
+  const int64_t ldV = L.rowLd;
+  const double* Cb = kV_.p + (size_t)(K1 - kc) * ldV;
+  multiDot(Cb, ldV, kc, r + L.row0, L.dotRows, kPartial_.p, kH_.p, 0, s, &launches_);
+  comm_.allReduceSum(kH_.p, (size_t)kc, s);
+  HY_CUDA(cudaMemsetAsync(kZ_.p, 0, ldV * sizeof(double), s));  // r may live in kZ_: read above, in stream order
+  multiAxpy(kRec_.p + (size_t)recU_ * K1 * ldV, ldV, kc, kH_.p, kZ_.p, L.rows, 1.0, s, &launches_);
+  HY_CUDA(cudaStreamSynchronize(s));
+  const double* upd = L.expand(kZ_.p);
+  if (right) {
+    L.M(upd, kW_.p);
+    upd = kW_.p;
+  }
+  axpby(1.0, upd, 1.0, kX_.p, L.len, s, &launches_);
+}
+
+// start of a cycle with kc recycled columns: v0 = (I - C C') r / beta', g = [C' r; beta' e1], the first kc columns
+// of the Hessenberg matrix D (no rotations).  false: beta' = 0, r lies in range(C).
+bool Engine::cycleStart(const KrylovLayout& L, double* base, int kc, const double* r, double* g, double* H, double* cs,
+                        double* sn, int m) {
+  cudaStream_t s = stream_;
+  const int64_t ldV = L.rowLd;
+  double* Vb = base + (size_t)kc * ldV;
+  double* dc = kH_.p;
+  double* dN = kH_.p + 2 * m + 2;
+  multiDot(base, ldV, kc, r + L.row0, L.dotRows, kPartial_.p, dc, 0, s, &launches_);
+  comm_.allReduceSum(dc, (size_t)kc, s);
+  axpby(1.0, r + L.row0, 0.0, Vb, L.rows, s, &launches_);
+  multiAxpy(base, ldV, kc, dc, Vb, L.rows, -1.0, s, &launches_);
+  multiDot(Vb, ldV, 1, Vb, L.dotRows, kPartial_.p, dN, 0, s, &launches_);
+  comm_.allReduceSum(dN, 1, s);
+  std::vector<double> h(2 * m + 3);
+  HY_CUDA(cudaMemcpyAsync(h.data(), kH_.p, (2 * m + 3) * sizeof(double), cudaMemcpyDeviceToHost, s));
+  HY_CUDA(cudaStreamSynchronize(s));
+  const double bp = std::sqrt(h[2 * m + 2]);
+  for (int i = 0; i < kc; ++i) {
+    g[i] = h[i];
+    for (int j = 0; j < kc; ++j) H[(size_t)i * m + j] = i == j ? recD_[i] : 0.0;
+    cs[i] = 1.0;
+    sn[i] = 0.0;
+  }
+  g[kc] = bp;
+  if (!(bp > 0.0)) return false;
+  scaleByInvNorm(Vb, dN, Vb, L.rows, s, &launches_);
+  return true;
+}
+
+// end of a cycle of kDone columns (kc recycled + the Arnoldi steps): the harmonic Ritz vectors of
+// Ghat' Ghat z = theta Ghat' (What' Vhat) z for the recK smallest |theta| give Ytilde = Vhat P, Ghat P = Q R,
+// C = What Q, U = Ytilde R^-1.  What = [C | v_0 .. v_p] (base, kDone + 1 vectors), Vhat = [Utilde | v_0 .. v_(p-1)].
+// Returns the new number of recycled columns; 0 when the Cholesky factorisation fails or Ghat P is rank deficient:
+// then no space is kept, and the next cycle is a plain GMRES cycle.
+int Engine::recycleUpdate(const KrylovLayout& L, int K1, int recK, double* base, int kc, int kDone,
+                          const std::vector<double>& G, int m) {
+  cudaStream_t s = stream_;
+  const int64_t ldV = L.rowLd;
+  const int mt = kDone, R1 = kDone + 1, pD = kDone - kc;
+  std::vector<double> Gh((size_t)R1 * mt, 0.0), WV((size_t)R1 * mt, 0.0);
+  for (int j = 0; j < kc; ++j) Gh[(size_t)j * R1 + j] = recD_[j];
+  for (int j = kc; j < mt; ++j) {
+    for (int i = 0; i <= j + 1; ++i) Gh[(size_t)j * R1 + i] = G[(size_t)i * m + j];
+    WV[(size_t)j * R1 + j] = 1.0;
+  }
+  if (kc) {  // What' Utilde: [C' U; V' U] D
+    const std::vector<double> wu = crossProducts(L, base, R1, kRec_.p + (size_t)recU_ * K1 * ldV, kc);
+    for (int j = 0; j < kc; ++j)
+      for (int i = 0; i < R1; ++i) WV[(size_t)j * R1 + i] = wu[(size_t)j * R1 + i] * recD_[j];
+  }
+  std::vector<double> A((size_t)mt * mt), B((size_t)mt * mt);
+  for (int j = 0; j < mt; ++j)
+    for (int i = 0; i < mt; ++i) {
+      double a = 0.0, b = 0.0;
+      for (int l = 0; l < R1; ++l) {
+        a += Gh[(size_t)i * R1 + l] * Gh[(size_t)j * R1 + l];
+        b += Gh[(size_t)i * R1 + l] * WV[(size_t)j * R1 + l];
+      }
+      A[(size_t)j * mt + i] = a;
+      B[(size_t)j * mt + i] = b;
+    }
+  const int kMax = std::min(K1, m - 1);  // at least one Arnoldi step per cycle
+  std::vector<double> P((size_t)mt * kMax);
+  int kn = 0;
+  auto drop = [&]() {
+    recDim_ = 0;
+    return 0;
+  };
+  if (hy_harmonic_ritz(mt, A.data(), B.data(), recK, kMax, P.data(), &kn) || kn == 0) return drop();
+  std::vector<double> GP((size_t)R1 * kn, 0.0), Q((size_t)R1 * kn), R((size_t)kn * kn);
+  for (int c = 0; c < kn; ++c)
+    for (int l = 0; l < mt; ++l) {
+      const double p = P[(size_t)c * mt + l];
+      if (p != 0.0)
+        for (int i = 0; i < R1; ++i) GP[(size_t)c * R1 + i] += Gh[(size_t)l * R1 + i] * p;
+    }
+  if (hy_qr(R1, kn, GP.data(), Q.data(), R.data(), 1e-12)) return drop();
+  const std::vector<double> Ri = upperInverse(R, kn);
+  // coefficients: [D P_u R^-1 (kc x kn) | P_v R^-1 (pD x kn) | Q (R1 x kn)], each column major
+  std::vector<double> coef((size_t)(mt + R1) * kn, 0.0);
+  double* cu = coef.data();
+  double* cv = cu + (size_t)kc * kn;
+  double* cq = cv + (size_t)pD * kn;
+  for (int c = 0; c < kn; ++c)
+    for (int l = 0; l < mt; ++l) {
+      double t = 0.0;
+      for (int q = 0; q <= c; ++q) t += P[(size_t)q * mt + l] * Ri[(size_t)c * kn + q];
+      if (l < kc) cu[(size_t)c * kc + l] = recD_[l] * t;
+      else cv[(size_t)c * pD + (l - kc)] = t;
+    }
+  std::copy(Q.begin(), Q.end(), cq);
+  HY_CUDA(cudaMemcpyAsync(kSmall_.p, coef.data(), coef.size() * sizeof(double), cudaMemcpyHostToDevice, s));
+  double* U = kRec_.p + (size_t)recU_ * K1 * ldV;
+  double* Un = kRec_.p + (size_t)(1 - recU_) * K1 * ldV;
+  const double* dcu = kSmall_.p;
+  const double* dcv = dcu + (size_t)kc * kn;
+  const double* dcq = dcv + (size_t)pD * kn;
+  if (kc) combine(U, ldV, kc, dcu, kc, Un, ldV, kn, L.rows, 0, s, &launches_);
+  combine(base + (size_t)kc * ldV, ldV, pD, dcv, pD, Un, ldV, kn, L.rows, kc ? 1 : 0, s, &launches_);
+  combine(base, ldV, R1, dcq, R1, U, ldV, kn, L.rows, 0, s, &launches_);  // C into the old U block
+  HY_CUDA(cudaMemcpyAsync(kV_.p + (size_t)(K1 - kn) * ldV, U, (size_t)kn * ldV * sizeof(double),
+                          cudaMemcpyDeviceToDevice, s));
+  HY_CUDA(cudaStreamSynchronize(s));  // coef is pageable host memory
+  recU_ = 1 - recU_;
+  recDim_ = kn;
+  recEpoch_ = opEpoch_;
+  recycleNorms(L, K1);
+  return kn;
+}
+
 void Engine::solve(const double* b, const double* T, double* x, double* S, VecEnds ends, int where, uint64_t seed,
                    hymls_b200_solve_info* info, double* hist, int histCap) {
   needDevice();
@@ -277,12 +486,20 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
   const bool explicitTest = it.get("Explicit Residual Test", false);
   const std::string impScaling = it.get("Implicit Residual Scaling", "Norm of Preconditioned Initial Residual");
   const std::string expScaling = it.get("Explicit Residual Scaling", "Norm of Initial Residual");
-  if (method != "GMRES" && method != "CG")
-    throw Error(HYMLS_B200_ERR_ARG, "Krylov Method '" + method + "' not supported (GMRES, CG)");
-  const bool gmres = method == "GMRES";
+  if (method != "GMRES" && method != "CG" && method != "GCRODR")
+    throw Error(HYMLS_B200_ERR_ARG, "Krylov Method '" + method + "' not supported (GMRES, CG, GCRODR)");
+  const bool gcrodr = method == "GCRODR";
+  const bool gmres = method == "GMRES" || gcrodr;  // GCRO-DR runs the GMRES cycle with the recycled space in front
   const bool single = gmres && singleBasis_;  // FP32 basis slots 1..m (readParameters refuses Single with CG)
   if (borderM_ && !gmres) throw Error(HYMLS_B200_ERR_UNSUPPORTED, "bordered solves use GMRES");
   const int m = std::max(1, std::min(numBlocks, maxIters));
+  // GCRO-DR: k recycled columns (k + 1 when a complex pair straddles k); only a GCRODR solve reads (and writes back)
+  // the parameter
+  const int recK = gcrodr ? it.get("Num Recycled Blocks", 5) : 0;
+  if (gcrodr && (recK < 1 || recK >= m))
+    throw Error(HYMLS_B200_ERR_ARG, "Num Recycled Blocks must be at least 1 and less than min(Num Blocks, Maximum "
+                                    "Iterations) = " + std::to_string(m));
+  const int K1 = gcrodr ? recK + 1 : 0;  // slots of C in front of the Arnoldi vectors
   const bool left = side == "Left", right = side == "Right";
   const KrylovLayout L = useDist() ? ownerLayout(left, right, ends) : replicatedLayout(left, right, ends);
   const int64_t n = L.len;
@@ -298,6 +515,12 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
   // the Krylov basis is workspace like the vectors above (grow-only, reused by later solves): a 40 GB cudaMalloc
   // does not belong into the event-timed iteration.  Each basis precision releases the storage of the other, so
   // switching a handle's mode frees that memory.
+  if (!gcrodr) {  // the recycled space of an earlier GCRODR list is gone (SetParameters dropped it): free its storage
+    kRec_.release();
+    kSmall_.release();
+    kPartialB_.release();
+    recDim_ = 0;
+  }
   if (single) {
     if (kV_.cap > (size_t)L.rowLd) kV_.release();
     kV_.alloc(L.rowLd);
@@ -306,7 +529,23 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
   } else if (gmres) {
     kVf_.release();
     kGs_.release();
-    kV_.alloc((size_t)(m + 1) * L.rowLd);
+    const size_t need = (size_t)(K1 + m + 1) * L.rowLd;
+    if (gcrodr) {  // a recycled space survives only on the same rows
+      if (recDim_ && (recRows_ != L.rows || recLd_ != L.rowLd || recRow0_ != L.row0 || recBorder_ != borderM_ ||
+                      recM_ != m || recCap_ != K1 || kV_.cap < need || kRec_.cap < 2 * (size_t)K1 * L.rowLd))
+        recDim_ = 0;
+      kRec_.alloc(2 * (size_t)K1 * L.rowLd);
+      kSmall_.alloc(3 * (size_t)(m + 2) * K1);
+      kPartialB_.alloc(blockDotPartial());
+      recRows_ = L.rows;
+      recLd_ = L.rowLd;
+      recRow0_ = L.row0;
+      recBorder_ = borderM_;
+      recM_ = m;
+      recCap_ = K1;
+      if (!recDim_) HY_CUDA(cudaMemsetAsync(kRec_.p, 0, kRec_.bytes(), stream_));
+    }
+    kV_.alloc(need);
   } else {
     kQ_.alloc(L.ld);
   }
@@ -382,7 +621,10 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
     }
   } else {
     const int64_t ldV = L.rowLd, nloc = L.rows, nDot = L.dotRows;
-    HY_CUDA(cudaMemsetAsync(kV_.p, 0, kV_.bytes(), s));
+    // GCRO-DR keeps C in the K1 slots in front of the Arnoldi vectors Vb; GMRES has K1 = 0
+    double* Vb = kV_.p + (size_t)K1 * ldV;
+    if (gcrodr && recDim_) HY_CUDA(cudaMemsetAsync(Vb, 0, (size_t)(m + 1) * ldV * sizeof(double), s));
+    else HY_CUDA(cudaMemsetAsync(kV_.p, 0, kV_.bytes(), s));
     if (single) {
       HY_CUDA(cudaMemsetAsync(kVf_.p, 0, kVf_.bytes(), s));
       HY_CUDA(cudaMemsetAsync(kGs_.p, 0, kGs_.bytes(), s));
@@ -398,6 +640,8 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
     double* dH1 = kH_.p;              // first Gram-Schmidt pass  (m+1)
     double* dH2 = kH_.p + (m + 1);    // second pass              (m+1)
     double* dNrm = kH_.p + 2 * m + 2; // ||w||^2
+    // GCRO-DR after a Compute: C = A^ U again (k operator applications, not iterations)
+    if (gcrodr && recDim_ && recEpoch_ != opEpoch_) rebuildRecycled(L, K1);
     const double r0norm = residual();
     double* r = kR_.p;
     if (left) {
@@ -417,22 +661,49 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
     const double impScale = scaleOf(impScaling), expScale = scaleOf(expScaling);
     double beta = pr0norm;
     double trueRes = r0norm;
+    // GCRO-DR state of this solve: kc recycled columns in use, C at Cb (the kc slots before Vb), U at Ub
+    int kc = 0;
+    std::vector<double> G;  // Ghat before the Givens rotations ((m+1) x m, row stride m)
+    if (gcrodr) {
+      G.assign((size_t)(m + 1) * m, 0.0);
+      kc = recDim_;
+      if (kc) {  // x += [M^-1] U C' r, then the residual of the new x (history[0] stays that of the initial guess)
+        history.push_back(beta / impScale);
+        recycleProject(L, K1, kc, r, right);
+        trueRes = residual();
+        r = kR_.p;
+        beta = trueRes;
+        if (left) {
+          L.M(kR_.p, kZ_.p);
+          r = kZ_.p;
+          beta = std::sqrt(dot(r, r));
+        }
+      }
+    }
     // HYMLS_B200_VERBOSE_SOLVE: wall time of the phases of every 50th Arnoldi step on stderr (synchronises the stream)
     static const bool verboseSolve = getenv("HYMLS_B200_VERBOSE_SOLVE") != nullptr;
     for (int restart = 0; restart <= maxRestarts; ++restart) {
-      if (restart == 0) history.push_back(beta / impScale);
+      if (restart == 0 && history.empty()) history.push_back(beta / impScale);
       lastRel = beta / impScale;
       if (beta == 0.0 || (lastRel <= tol && !explicitTest)) {  // a zero residual cannot be normalised
         converged = true;
         break;
       }
-      axpby(1.0 / beta, r + L.row0, 0.0, kV_.p, nloc, s, &launches_);  // v0 = r / beta (this rank's rows)
       std::fill(g.begin(), g.end(), 0.0);
-      g[0] = beta;
-      int kDone = 0;
-      for (int k = 0; k < m && iters < maxIters; ++k) {
-        const double* vk = !single ? kV_.p + (size_t)k * ldV : k == 0 ? v0 : vin;
-        double* w = single ? wS : kV_.p + (size_t)(k + 1) * ldV;
+      // basis of the cycle: [C | v_0 v_1 ...] from `base`; column k >= kc of the Hessenberg matrix belongs to v_(k-kc)
+      double* base = Vb - (size_t)kc * ldV;
+      bool empty = false;
+      if (kc) {  // v0 = (I - C C') r / beta', g = [C' r; beta' e1]; the first kc columns of Ghat are D (triangular)
+        empty = !cycleStart(L, base, kc, r, g.data(), H.data(), cs.data(), sn.data(), m);
+        if (empty) recycleProject(L, K1, kc, r, right);  // r lies in range(C): the projection solves
+      } else {
+        axpby(1.0 / beta, r + L.row0, 0.0, Vb, nloc, s, &launches_);  // v0 = r / beta (this rank's rows)
+        g[0] = beta;
+      }
+      int kDone = kc;
+      for (int k = kc; k < m && iters < maxIters && !empty; ++k) {
+        const double* vk = !single ? base + (size_t)k * ldV : k == 0 ? v0 : vin;
+        double* w = single ? wS : base + (size_t)(k + 1) * ldV;
         const bool lapIt = verboseSolve && comm_.rank() == 0 && (k % 50) == 20;
         auto tl = std::chrono::steady_clock::now();
         auto lap = [&](const char* what) {
@@ -455,14 +726,14 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
             multiDot(v0, ldV, 1, w, nDot, kPartial_.p, dh, 0, s, &launches_);
             multiDot(Vf, ldV, k, w, nDot, kPartial_.p, dh + 1, 0, s, &launches_);
           } else {
-            multiDot(kV_.p, ldV, k + 1, w, nDot, kPartial_.p, dh, 0, s, &launches_);
+            multiDot(base, ldV, k + 1, w, nDot, kPartial_.p, dh, 0, s, &launches_);
           }
           comm_.allReduceSum(dh, (size_t)(k + 1), s);
           if (single) {
             multiAxpy(v0, ldV, 1, dh, w, nloc, -1.0, s, &launches_);
             multiAxpy(Vf, ldV, k, dh + 1, w, nloc, -1.0, s, &launches_);
           } else {
-            multiAxpy(kV_.p, ldV, k + 1, dh, w, nloc, -1.0, s, &launches_);
+            multiAxpy(base, ldV, k + 1, dh, w, nloc, -1.0, s, &launches_);
           }
         }
         multiDot(w, ldV, 1, w, nDot, kPartial_.p, dNrm, 0, s, &launches_);
@@ -481,7 +752,11 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
         for (int i = 0; i <= k; ++i) colNorm = std::hypot(colNorm, hbuf[i] + hbuf[m + 1 + i]);
         const bool breakdown = !(hn > 1e-300) || hn <= 1e-15 * colNorm;
         H[(size_t)(k + 1) * m + k] = breakdown ? 0.0 : hn;
-        for (int i = 0; i < k; ++i) {
+        if (gcrodr) {  // the unrotated column for the harmonic Ritz problem; a breakdown leaves no finite v_(k+1)
+          for (int i = 0; i <= k + 1; ++i) G[(size_t)i * m + k] = H[(size_t)i * m + k];
+          if (breakdown) HY_CUDA(cudaMemsetAsync(w, 0, ldV * sizeof(double), s));
+        }
+        for (int i = kc; i < k; ++i) {
           const double t = cs[i] * H[(size_t)i * m + k] + sn[i] * H[(size_t)(i + 1) * m + k];
           H[(size_t)(i + 1) * m + k] = -sn[i] * H[(size_t)i * m + k] + cs[i] * H[(size_t)(i + 1) * m + k];
           H[(size_t)i * m + k] = t;
@@ -499,7 +774,7 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
         history.push_back(lastRel);
         if (lastRel <= tol || breakdown) break;
       }
-      if (kDone > 0) {
+      if (kDone > kc) {
         // y = triu(H)^-1 g ; x += [M^-1] V y
         std::vector<double> y(kDone);
         for (int i = kDone - 1; i >= 0; --i) {
@@ -513,7 +788,13 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
           multiAxpy(v0, ldV, 1, dH1, kZ_.p, nloc, 1.0, s, &launches_);
           multiAxpy(Vf, ldV, kDone - 1, dH1 + 1, kZ_.p, nloc, 1.0, s, &launches_);
         } else {
-          multiAxpy(kV_.p, ldV, kDone, dH1, kZ_.p, nloc, 1.0, s, &launches_);
+          multiAxpy(Vb, ldV, kDone - kc, dH1 + kc, kZ_.p, nloc, 1.0, s, &launches_);
+          if (kc) {  // + Utilde y_u = U (D y_u)
+            std::vector<double> yu(kc);
+            for (int i = 0; i < kc; ++i) yu[i] = y[i] * recD_[i];
+            HY_CUDA(cudaMemcpyAsync(dH2, yu.data(), kc * sizeof(double), cudaMemcpyHostToDevice, s));
+            multiAxpy(kRec_.p + (size_t)recU_ * K1 * ldV, ldV, kc, dH2, kZ_.p, nloc, 1.0, s, &launches_);
+          }
         }
         HY_CUDA(cudaStreamSynchronize(s));
         const double* upd = L.expand(kZ_.p);
@@ -523,6 +804,8 @@ void Engine::solve(const double* b, const double* T, double* x, double* S, VecEn
         }
         axpby(1.0, upd, 1.0, kX_.p, n, s, &launches_);
       }
+      // GCRO-DR: the harmonic Ritz vectors of this cycle become the recycled space of the next cycle and solve
+      if (gcrodr && kDone > kc && kDone > recK) kc = recycleUpdate(L, K1, recK, base, kc, kDone, G, m);
       trueRes = residual();
       r = kR_.p;
       beta = trueRes;

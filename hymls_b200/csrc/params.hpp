@@ -28,6 +28,7 @@ class ParameterList {
   };
 
   bool isParameter(const std::string& n) const { return vals_.count(n) != 0; }
+  Kind kindOf(const std::string& n) const { return vals_.at(n).kind; }  // the parameter must exist
   bool isSublist(const std::string& n) const { return subs_.count(n) != 0; }
   ParameterList& sublist(const std::string& n) {
     auto it = subs_.find(n);

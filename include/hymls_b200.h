@@ -186,6 +186,12 @@ int hymls_b200_apply_matrix(hymls_b200_t* h, const double* x, double* y, int whe
  * orthogonalisation, but different iterates and possibly more iterations.  A Single cycle counts as converged only
  * when the residual recomputed in FP64 also meets the tolerance in the implicit scaling, so info->converged = 1 always
  * means that the FP64 residual met it.
+ * "Krylov Method" = "GCRODR" runs GCRO-DR (Parks et al. 2006; Belos GCRODR): every cycle of "Num Blocks" = m
+ * directions keeps k = "Num Recycled Blocks" (default 5, 1 <= k < m) harmonic Ritz vectors U_k with C_k = A^ U_k,
+ * A^ the (preconditioned) operator, and the next cycle runs m - k Arnoldi steps orthogonal to C_k.  The space belongs
+ * to the handle: it carries over into the next hymls_b200_solve / _solve_dist / _solve_map, which first projects the
+ * initial residual onto C_k.  After a Compute (new matrix or border values) C_k = A^ U_k is rebuilt with k operator
+ * applications that are not counted as iterations; Initialize, SetParameters and a change of the border size drop it.
  */
 typedef struct {
   int iterations;
@@ -293,7 +299,13 @@ typedef struct {
                                    entries, or n / ranks rounded up; the owned rows + border rounded up to 8 on the owner
                                    distribution): 8 (m + 1) rowLd with "Krylov Basis Precision" = "Double", 4 m rowLd + 8 rowLd
                                    (FP32 slots 1..m, FP64 first vector) with "Single".  Storage is grow-only within one mode:
-                                   the largest m so far counts; a solve in the other mode releases it */
+                                   the largest m so far counts; a solve in the other mode releases it.  A "GCRODR" solve with
+                                   k = Num Recycled Blocks adds the recycled space: 8 (m + 1 + 3 (k + 1)) rowLd, i.e. the
+                                   Arnoldi vectors, k + 1 slots of C before them, and U with the restart's scratch (k + 1
+                                   columns each; k + 1 keeps a complex harmonic Ritz pair whole) */
+  int64_t krylov_recycle_dim;   /* columns of the recycled GCRO-DR space U_k / C_k the handle holds (k, or k + 1 when a complex
+                                   pair straddles k; 0: none).  It persists across solves and is dropped by Initialize,
+                                   SetParameters and a change of the border size */
 } hymls_b200_stats;
 int hymls_b200_get_stats(hymls_b200_t* h, hymls_b200_stats* st);
 
